@@ -2,7 +2,7 @@
 """bench.py - SDF decoder queries/s on N B200s (BASELINE.json metric), plus roofline, accuracy against the frozen
 oracle, end-to-end (host buffers through the C ABI) and a CPU-oracle baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N = 1 - a step = decode_grid(z, 256): BASELINE.json configs[1], one latent on a 256^3 grid (16,777,216 queries), bf16
 operands / fp32 accumulate, fused tcgen05 kernel.  The same step is also timed with fp16 operands (the precision that meets
@@ -46,6 +46,18 @@ DDPM_FLOP_PER_LATENT_STEP = 2 * (512 * 1024 + 3 * 1024 * 1024 + 1024 * 256)   # 
 METRIC = "sdf_decoder_queries_per_s"
 UNIT = "queries/s"
 REF_BUDGET_S = 15.0
+DUMP_DRAWS = 1 << 22            # seeded draws per dumped array: ~4 M distinct elements, at most 16 MiB of float32
+
+
+def dump_sample(t, seed: int):
+    """--dump-outputs: a fixed, seeded sample of `t`'s elements (flat order) as float32, so that two builds can be compared
+    element for element without writing a whole 256^3 / 512^3 grid."""
+    import numpy as np
+    import torch
+    drawn = np.zeros(t.numel(), dtype=bool)
+    drawn[np.random.RandomState(seed).randint(0, t.numel(), DUMP_DRAWS, dtype=np.int64)] = True
+    idx = np.flatnonzero(drawn)                                # distinct, in ascending order
+    return t.reshape(-1)[torch.from_numpy(idx).to(t.device)].float().cpu().numpy()
 
 
 def read_peaks():
@@ -287,8 +299,13 @@ def main():
     ap.add_argument("--no-ddpm", action="store_true", help="skip the latent-DDPM leg (second half of the metric)")
     ap.add_argument("--no-vjp", action="store_true", help="skip the latent-gradient leg (SURVEY 8f row N4)")
     ap.add_argument("--no-train", action="store_true", help="skip the training-step legs (SURVEY 8f row N4)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the headline step returned in its last timed step to DIR/<name>.npy (float32, rank 0): a fixed "
+                         "seeded sample of the sdf grid, and with the sharded 512^3 headline (N > 1) of its unpacked sign-change mask")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU arm's outputs; the reference arm has none to compare")
         return run_reference(args)
 
     # stdout carries exactly one JSON line: anything libraries print there (NCCL's version banner, ...) goes to stderr
@@ -337,7 +354,8 @@ def main():
         return float(t.item())
 
     def time_grid(prec: str, steps: int, warm: int, clk=None):
-        """`steps` timed decode_grid(z, 256) calls: (sum of per-step event times, max over ranks; mean kernel ms)."""
+        """`steps` timed decode_grid(z, 256) calls: (sum of per-step event times, max over ranks; mean kernel ms; the sdf
+        of the last step)."""
         out = torch.empty((RES, RES, RES), dtype=torch.float32, device=dev)
         for _ in range(warm):
             dec.decode_grid(z, RES, out=out, precision=prec)
@@ -353,19 +371,22 @@ def main():
             kms.append(dec.last_kernel_ms())                       # events around the fused kernel itself; raises on a watchdog trip
         barrier()
         total = max_over_ranks(sum(a.elapsed_time(b) for a, b in ev))
-        del out
-        return total, statistics.mean(kms)
+        return total, statistics.mean(kms), out
 
     peaks = read_peaks()
     headline5 = world > 1 and not args.no_config5
     line = {}
+    dumps = {}                                                     # --dump-outputs: name -> sampled float32 array
 
     # ---- decode_grid(z, 256) per rank: the N = 1 headline; at N > 1 the collective-free weak-scaling number
     with ClockSampler(local) as clk1:
         t_wall0 = time.perf_counter()
         Kg = K if not headline5 else max(3, min(K, 5))
-        total_ms, k_ms = time_grid(args.precision, Kg, W)
+        total_ms, k_ms, sdf_last = time_grid(args.precision, Kg, W)
         t_wall = time.perf_counter() - t_wall0
+    if args.dump_outputs and rank == 0 and not headline5:
+        dumps["sdf"] = dump_sample(sdf_last, 0)
+    del sdf_last
     grid_value = world * QUERIES * Kg / (total_ms * 1e-3)
     achieved = QUERIES * FLOP_TENSOR_PER_QUERY / (k_ms * 1e-3) / 1e12
     traffic, traffic_src = read_ncu_traffic()
@@ -383,7 +404,7 @@ def main():
     if not args.no_second_precision:
         other = "fp16" if args.precision == "bf16" else "bf16"
         Ks = max(3, min(K, 10))
-        t2, k2 = time_grid(other, Ks, 2)
+        t2, k2, _ = time_grid(other, Ks, 2)
         a2 = QUERIES * FLOP_TENSOR_PER_QUERY / (k2 * 1e-3) / 1e12
         second = {"dtype": other, "value": world * QUERIES * Ks / (t2 * 1e-3), "unit": UNIT, "steps": Ks, "ms_per_step": t2 / Ks,
                   "kernel_ms": k2, "achieved_tflops": a2, "frac_of_burst_peak": a2 / peaks["burst"],
@@ -464,6 +485,9 @@ def main():
                 ev[i][1].synchronize()
             barrier()
         dec.check()
+        if args.dump_outputs and rank == 0:          # s5 / m5 of the push path are views: sampled before the next sharded decode
+            dumps["sdf"] = dump_sample(s5, 0)
+            dumps["mask"] = dump_sample(pkg.unpack_mask_blocks(m5, RES5) if push_path else m5, 1)
         step5 = [a.elapsed_time(b) for a, b in ev]
         total5 = max_over_ranks(sum(step5))
         med5 = max_over_ranks(statistics.median(step5))
@@ -770,6 +794,10 @@ def main():
             line["cpu_baseline"] = cpu_base
         elif world > 1:
             line["cpu_baseline_note"] = "timed on rank 0 at N = 1 only (see the N = 1 line)"
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dumps.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         sys.stdout.flush()
         os.write(json_fd, (json.dumps(line) + "\n").encode())
     if world > 1:

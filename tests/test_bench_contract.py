@@ -1,9 +1,13 @@
 """bench.py's reference arm (the CPU oracle on the host cores) runs without a GPU: one short step here guards the
-JSON contract of that arm; the keys of the GPU arm's line are checked on a saved line from profiles/."""
+JSON contract of that arm; the keys of the GPU arm's line are checked on a saved line from profiles/, and its --dump-outputs
+files on the GPU."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BASE_KEYS = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
@@ -64,3 +68,29 @@ def test_round2_lines_have_the_contract_keys():
     assert abs(m["value"] - 512 ** 3 / (c5["ms_per_step"] * 1e-3)) < 1e-3 * m["value"]
     assert c5["ms_per_step"] < 50 and c5["second_precision"]["dtype"] == "fp16" and c5["second_precision"]["ms_per_step"] < 50
     assert "512" in m["config"]["workload"] and m["e2e"]["d2h_bytes_per_step"] > 0
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_step(pkg, tmp_path):
+    """--dump-outputs DIR: the seeded sample of the headline decode_grid(z, 256) written after --steps timed steps is the same
+    on a second run with another step count, and is what the package's own decode of the benchmark's latent returns."""
+    import torch
+    import bench
+    legs_off = ["--no-cpu-baseline", "--no-accuracy", "--no-second-precision", "--no-config4", "--no-ddpm", "--no-vjp", "--no-train"]
+    dumped = []
+    for steps in (2, 3):
+        out_dir = tmp_path / f"steps{steps}"
+        proc = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1",
+                               "--dump-outputs", str(out_dir), *legs_off], capture_output=True, text=True, timeout=600, cwd=ROOT)
+        assert proc.returncode == 0, proc.stderr[-2000:]
+        lines = [ln for ln in proc.stdout.splitlines() if ln.strip()]
+        assert len(lines) == 1 and json.loads(lines[0])["steps"] == steps
+        assert sorted(os.listdir(out_dir)) == ["sdf.npy"]
+        assert sum(os.path.getsize(out_dir / f) for f in os.listdir(out_dir)) <= 64_000_000
+        dumped.append(np.load(out_dir / "sdf.npy"))
+    assert dumped[0].dtype == np.float32 and dumped[0].size > 3_000_000
+    assert np.array_equal(dumped[0], dumped[1])
+    dec = pkg.Decoder(pkg.synthetic.decoder_params(), device="cuda:0", precision="bf16")
+    sdf = dec.decode_grid(torch.from_numpy(pkg.synthetic.latent(0)).cuda(), 256)
+    assert np.array_equal(dumped[0], bench.dump_sample(sdf, 0))
+    dec.close()
