@@ -177,27 +177,6 @@ int sdfb_mc_weld_count(const int64_t* edge_keys_dev, int64_t n_triangles, int re
 int sdfb_mc_weld_fill(const float* triangles_dev, const int64_t* edge_keys_dev, int64_t n_triangles, int res, const void* workspace_dev,
                       float* vertices_dev, int64_t* faces_dev, void* stream);
 
-/* ---- sparse extraction (SURVEY.md 8f row N2): decode only near the surface ---------------------------
- * The res^3 grid is cut into blocks of `block`^3 cells (nb = ceil((res-1)/block) per axis; the last block
- * may be ragged).  1) sdfb_sparse_corner_points: xyz of the (nb+1)^3 block corners -> decode them with
- * sdfb_decode_points.  2) sdfb_sparse_select_blocks: keeps a block if its 8 corner values differ in sign or
- * one of them is within `tau` of zero (tau = L * block * h * sqrt(3) / 2 is exact for an L-Lipschitz field,
- * h = 2 / (res - 1)); ids ascending, id = (bz*nb + by)*nb + bx; returns their number (synchronises).
- * 3) sdfb_sparse_block_points: xyz of the (block+1)^3 nodes of every kept block -> decode them.
- * 4) sdfb_mc_blocks_count / _generate: marching cubes over those fields [n_blocks][(block+1)^3]: the
- * same triangles, bit for bit, as the dense extraction wherever the kept blocks cover the surface. */
-int sdfb_sparse_corner_points(int res, int block, float* xyz_dev, void* stream);
-int sdfb_sparse_select_workspace_bytes(int res, int block, size_t* bytes);
-int sdfb_sparse_select_blocks(const float* corner_sdf_dev, int res, int block, float tau, int32_t* block_ids_dev,
-                              void* workspace_dev, size_t workspace_bytes, int64_t* n_blocks_host, void* stream);
-int sdfb_sparse_block_points(int res, int block, const int32_t* block_ids_dev, int64_t n_blocks, float* xyz_dev,
-                             void* stream);
-int sdfb_mc_blocks_workspace_bytes(int block, int64_t n_blocks, size_t* bytes);
-int sdfb_mc_blocks_count(const float* fields_dev, const int32_t* block_ids_dev, int64_t n_blocks, int res, int block,
-                         void* workspace_dev, size_t workspace_bytes, int64_t* n_triangles_host, void* stream);
-int sdfb_mc_blocks_generate(const float* fields_dev, const int32_t* block_ids_dev, int64_t n_blocks, int res, int block,
-                            const void* workspace_dev, float* triangles_dev, int64_t* edge_keys_dev, void* stream);
-
 /* Synchronises `stream` and reports (once) a watchdog trip of any launch made on this context. */
 int sdfb_decoder_check(sdfb_decoder* dec, void* stream);
 /* Per-wait timeout of the in-kernel watchdog (default 2 s).  Test hook: a few nanoseconds make the next launch fail. */

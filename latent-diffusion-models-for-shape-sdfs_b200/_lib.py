@@ -43,13 +43,6 @@ SIGNATURES = {
     "sdfb_mc_workspace_bytes": (_i, [_i, _i, _i, C.POINTER(_sz)]),
     "sdfb_mc_count": (_i, [_vp, _vp, _i, _i, _i, _vp, _sz, C.POINTER(_i64), _vp]),
     "sdfb_mc_generate": (_i, [_vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
-    "sdfb_sparse_corner_points": (_i, [_i, _i, _vp, _vp]),
-    "sdfb_sparse_select_workspace_bytes": (_i, [_i, _i, C.POINTER(_sz)]),
-    "sdfb_sparse_select_blocks": (_i, [_vp, _i, _i, C.c_float, _vp, _vp, _sz, C.POINTER(_i64), _vp]),
-    "sdfb_sparse_block_points": (_i, [_i, _i, _vp, _i64, _vp, _vp]),
-    "sdfb_mc_blocks_workspace_bytes": (_i, [_i, _i64, C.POINTER(_sz)]),
-    "sdfb_mc_blocks_count": (_i, [_vp, _vp, _i64, _i, _i, _vp, _sz, C.POINTER(_i64), _vp]),
-    "sdfb_mc_blocks_generate": (_i, [_vp, _vp, _i64, _i, _i, _vp, _vp, _vp, _vp]),
     "sdfb_decode_sparse_field": (_i, [_vp, _vp, _i, C.c_float, C.c_float, C.c_float, C.c_float, _vp, _vp, _i, _vp, _vp]),
     "sdfb_decode_debug_pass": (_i, [_vp, _vp, _i, _i, _vp, _i, _vp]),
     "sdfb_decoder_last_kernel_ms": (_i, [_vp, C.POINTER(C.c_float)]),

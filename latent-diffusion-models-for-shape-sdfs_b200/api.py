@@ -319,75 +319,17 @@ class Decoder:
         st.update(dense_queries=res ** 3, lipschitz_level1=stats[6] * 1e-6, lipschitz_level2=stats[7] * 1e-6)
         return sdf, signs, st
 
-    def extract_surface_sparse(self, latent, res: int, block: int = 8, lipschitz: float | None = None,
-                               precision: str | None = None, return_stats: bool = False, indexed: bool = False,
-                               method: str = "hier", local_floor: float = 0.0):
-        """The zero level set on the res^3 grid WITHOUT decoding the whole grid.
-
-        ``method="hier"`` (default): two-level refinement (``decode_sparse_field``), every node decoded at most once, then
-        the DENSE marching-cubes kernels over the complete sign bit-planes - with a valid Lipschitz bound the triangle soup
-        equals ``extract_surface``'s bit for bit, order included.  ``local_floor`` in (0, 1] lets level 2 use every 8^3 block's
-        own slope estimate (never less than that fraction of the global one): a thinner band, fewer queries, less margin.
-
-        ``method="blocks"`` (round 1): decode the corners of
-        `block`^3-cell blocks, keep the blocks whose corners straddle zero or come within
-        tau = L * block * h * sqrt(3) / 2 of it (h = 2 / (res - 1)), decode only their nodes and run marching
-        cubes on them.  With a valid Lipschitz bound L the triangles are those of the dense extraction, bit for
-        bit (the order differs).  ``lipschitz=None`` estimates L from the block-corner values (largest difference
-        quotient along block edges, times 2)."""
-        if method == "hier":
-            sdf, signs, st = self.decode_sparse_field(latent, res, lipschitz=lipschitz, precision=precision, local_floor=local_floor)
-            out = extract_surface(sdf, res, 0, sign_words=signs, indexed=indexed)
-            self.check()
-            return (out, st) if return_stats else out
-        if method != "blocks":
-            raise ValueError("method must be 'hier' or 'blocks'")
-        lib = self._lib
-        nb = (res - 1 + block - 1) // block
-        st = _stream_ptr(self.device.index)
-        with torch.cuda.device(self.device):
-            corners = torch.empty(((nb + 1) ** 3, 3), dtype=torch.float32, device=self.device)
-            check(lib.sdfb_sparse_corner_points(res, block, corners.data_ptr(), st))
-            cs = self(latent, corners, precision=precision)
-            h = 2.0 / (res - 1)
-            if lipschitz is None:
-                g = cs.view(nb + 1, nb + 1, nb + 1)
-                dq = max(float((g[1:] - g[:-1]).abs().max()), float((g[:, 1:] - g[:, :-1]).abs().max()),
-                         float((g[:, :, 1:] - g[:, :, :-1]).abs().max())) / (block * h)
-                lipschitz = 2.0 * dq
-            tau = float(lipschitz) * block * h * (3.0 ** 0.5) / 2.0
-            nbytes = C.c_size_t()
-            check(lib.sdfb_sparse_select_workspace_bytes(res, block, C.byref(nbytes)))
-            ws = torch.empty((nbytes.value,), dtype=torch.uint8, device=self.device)
-            ids = torch.empty((nb ** 3,), dtype=torch.int32, device=self.device)
-            nblk = C.c_int64()
-            check(lib.sdfb_sparse_select_blocks(cs.data_ptr(), res, block, C.c_float(tau), ids.data_ptr(), ws.data_ptr(),
-                                                nbytes.value, C.byref(nblk), st))
-            n = nblk.value
-            per = (block + 1) ** 3
-            tris = torch.empty((0, 3, 3), dtype=torch.float32, device=self.device)
-            keys = torch.empty((0, 3), dtype=torch.int64, device=self.device)
-            if n:
-                pts = torch.empty((n * per, 3), dtype=torch.float32, device=self.device)
-                check(lib.sdfb_sparse_block_points(res, block, ids.data_ptr(), n, pts.data_ptr(), st))
-                fields = self(latent, pts, precision=precision)
-                check(lib.sdfb_mc_blocks_workspace_bytes(block, n, C.byref(nbytes)))
-                ws2 = torch.empty((nbytes.value,), dtype=torch.uint8, device=self.device)
-                ntri = C.c_int64()
-                check(lib.sdfb_mc_blocks_count(fields.data_ptr(), ids.data_ptr(), n, res, block, ws2.data_ptr(), nbytes.value,
-                                               C.byref(ntri), st))
-                tris = torch.empty((ntri.value, 3, 3), dtype=torch.float32, device=self.device)
-                keys = torch.empty((ntri.value, 3), dtype=torch.int64, device=self.device)
-                if ntri.value:
-                    check(lib.sdfb_mc_blocks_generate(fields.data_ptr(), ids.data_ptr(), n, res, block, ws2.data_ptr(),
-                                                      tris.data_ptr(), keys.data_ptr() if indexed else None, st))
-        self.check()                # the counts above already synchronised the stream
-        if indexed:
-            tris = weld(tris, keys, res)
-        if return_stats:
-            return tris, {"blocks": n, "blocks_total": nb ** 3, "queries": (nb + 1) ** 3 + n * per, "dense_queries": res ** 3,
-                          "tau": tau, "lipschitz": float(lipschitz)}
-        return tris
+    def extract_surface_sparse(self, latent, res: int, lipschitz: float | None = None, precision: str | None = None,
+                               return_stats: bool = False, indexed: bool = False, local_floor: float = 0.0):
+        """The zero level set on the res^3 grid WITHOUT decoding the whole grid: two-level refinement
+        (``decode_sparse_field``), every node decoded at most once, then the DENSE marching-cubes kernels over the complete
+        sign bit-planes - with a valid Lipschitz bound the triangle soup equals ``extract_surface``'s bit for bit, order
+        included.  ``local_floor`` in (0, 1] lets level 2 use every 8^3 block's own slope estimate (never less than that
+        fraction of the global one): a thinner band, fewer queries, less margin."""
+        sdf, signs, st = self.decode_sparse_field(latent, res, lipschitz=lipschitz, precision=precision, local_floor=local_floor)
+        out = extract_surface(sdf, res, 0, sign_words=signs, indexed=indexed)
+        self.check()
+        return (out, st) if return_stats else out
 
     def decode_grid_batch(self, latents, res: int, precision: str | None = None, out: torch.Tensor | None = None) -> torch.Tensor:
         """sdf [B, res, res, res] for latents [B,256] (independent shapes, one C call)."""

@@ -1001,10 +1001,24 @@ McLayout mc_layout(long long nodes, long long cells) {
   return L;
 }
 
-int mc_count_impl(const float* sdf_dev, const uint32_t* sign_bits_dev, const McGeom& g, void* workspace_dev,
-                  size_t workspace_bytes, int64_t* n_triangles_host, cudaStream_t st) {
+}  // namespace
+
+int sdfb_mc_workspace_bytes(int nz, int ny, int nx, size_t* bytes) {
+  if (!bytes) return fail(SDFB_E_INVALID, "null argument");
+  if (nz < 2 || ny < 2 || nx < 2) return fail(SDFB_E_INVALID, "the field must have at least 2 nodes per axis");
+  const McGeom g = mc_dense_geom(nz, ny, nx, nx, 0);
+  *bytes = mc_layout(g.total_nodes, g.total_cells).total;
+  return SDFB_OK;
+}
+
+int sdfb_mc_count(const float* sdf_dev, const uint32_t* sign_bits_dev, int nz, int ny, int nx, void* workspace_dev,
+                  size_t workspace_bytes, int64_t* n_triangles_host, void* stream) {
+  if (!sdf_dev || !workspace_dev || !n_triangles_host) return fail(SDFB_E_INVALID, "null argument");
+  if (nz < 2 || ny < 2 || nx < 2) return fail(SDFB_E_INVALID, "the field must have at least 2 nodes per axis");
+  const McGeom g = mc_dense_geom(nz, ny, nx, nx, 0);
   const McLayout L = mc_layout(g.total_nodes, g.total_cells);
   if (workspace_bytes < L.total) return fail(SDFB_E_INVALID, "workspace holds %zu bytes, %zu needed", workspace_bytes, L.total);
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
   uint8_t* ws = static_cast<uint8_t*>(workspace_dev);
   unsigned int* bits = reinterpret_cast<unsigned int*>(ws + L.off_bits);
   unsigned int* groups = reinterpret_cast<unsigned int*>(ws + L.off_groups);
@@ -1020,38 +1034,17 @@ int mc_count_impl(const float* sdf_dev, const uint32_t* sign_bits_dev, const McG
   return SDFB_OK;
 }
 
-int mc_generate_impl(const float* sdf_dev, const McGeom& g, const void* workspace_dev, float* triangles_dev, long long* keys_dev,
-                     cudaStream_t st) {
-  const McLayout L = mc_layout(g.total_nodes, g.total_cells);
-  const uint8_t* ws = static_cast<const uint8_t*>(workspace_dev);
-  CU_TRY(launch_mc_generate(sdf_dev, reinterpret_cast<const unsigned int*>(ws + L.off_bits),
-                            reinterpret_cast<const unsigned int*>(ws + L.off_groups), g, triangles_dev, keys_dev, st));
-  return SDFB_OK;
-}
-}  // namespace
-
-int sdfb_mc_workspace_bytes(int nz, int ny, int nx, size_t* bytes) {
-  if (!bytes) return fail(SDFB_E_INVALID, "null argument");
-  if (nz < 2 || ny < 2 || nx < 2) return fail(SDFB_E_INVALID, "the field must have at least 2 nodes per axis");
-  const McGeom g = mc_dense_geom(nz, ny, nx, nx, 0);
-  *bytes = mc_layout(g.total_nodes, g.total_cells).total;
-  return SDFB_OK;
-}
-
-int sdfb_mc_count(const float* sdf_dev, const uint32_t* sign_bits_dev, int nz, int ny, int nx, void* workspace_dev,
-                  size_t workspace_bytes, int64_t* n_triangles_host, void* stream) {
-  if (!sdf_dev || !workspace_dev || !n_triangles_host) return fail(SDFB_E_INVALID, "null argument");
-  if (nz < 2 || ny < 2 || nx < 2) return fail(SDFB_E_INVALID, "the field must have at least 2 nodes per axis");
-  return mc_count_impl(sdf_dev, sign_bits_dev, mc_dense_geom(nz, ny, nx, nx, 0), workspace_dev, workspace_bytes, n_triangles_host,
-                       static_cast<cudaStream_t>(stream));
-}
-
 int sdfb_mc_generate(const float* sdf_dev, int nz, int ny, int nx, int res, int z0, const void* workspace_dev,
                      float* triangles_dev, int64_t* edge_keys_dev, void* stream) {
   if (!sdf_dev || !workspace_dev || !triangles_dev) return fail(SDFB_E_INVALID, "null argument");
   if (nz < 2 || ny < 2 || nx < 2 || res < 2 || z0 < 0) return fail(SDFB_E_INVALID, "bad field shape");
-  return mc_generate_impl(sdf_dev, mc_dense_geom(nz, ny, nx, res, z0), workspace_dev, triangles_dev,
-                          reinterpret_cast<long long*>(edge_keys_dev), static_cast<cudaStream_t>(stream));
+  const McGeom g = mc_dense_geom(nz, ny, nx, res, z0);
+  const McLayout L = mc_layout(g.total_nodes, g.total_cells);
+  const uint8_t* ws = static_cast<const uint8_t*>(workspace_dev);
+  CU_TRY(launch_mc_generate(sdf_dev, reinterpret_cast<const unsigned int*>(ws + L.off_bits),
+                            reinterpret_cast<const unsigned int*>(ws + L.off_groups), g, triangles_dev,
+                            reinterpret_cast<long long*>(edge_keys_dev), static_cast<cudaStream_t>(stream)));
+  return SDFB_OK;
 }
 
 // ---- welding the soup into an indexed mesh ----
@@ -1086,82 +1079,6 @@ int sdfb_mc_weld_fill(const float* triangles_dev, const int64_t* edge_keys_dev, 
                              static_cast<const uint8_t*>(workspace_dev) + 256, vertices_dev, reinterpret_cast<long long*>(faces_dev),
                              static_cast<cudaStream_t>(stream)));
   return SDFB_OK;
-}
-
-// ---- sparse extraction: coarse block corners -> block selection -> nodes of the selected blocks -> marching cubes ----
-int sdfb_sparse_corner_points(int res, int block, float* xyz_dev, void* stream) {
-  if (!xyz_dev) return fail(SDFB_E_INVALID, "null argument");
-  if (res < 2 || block < 1 || block > 64) return fail(SDFB_E_INVALID, "bad res or block size");
-  const int nb = (res - 1 + block - 1) / block;
-  CU_TRY(launch_block_corner_points(res, block, nb, xyz_dev, static_cast<cudaStream_t>(stream)));
-  return SDFB_OK;
-}
-
-int sdfb_sparse_select_workspace_bytes(int res, int block, size_t* bytes) {
-  if (!bytes) return fail(SDFB_E_INVALID, "null argument");
-  if (res < 2 || block < 1 || block > 64) return fail(SDFB_E_INVALID, "bad res or block size");
-  const long long nb = (res - 1 + block - 1) / block, total = nb * nb * nb;
-  *bytes = static_cast<size_t>((total + 255) / 256 * 256) + static_cast<size_t>(total) * 4 + 256 + block_select_temp_bytes(total) + 256;
-  return SDFB_OK;
-}
-
-int sdfb_sparse_select_blocks(const float* corner_sdf_dev, int res, int block, float tau, int32_t* block_ids_dev,
-                              void* workspace_dev, size_t workspace_bytes, int64_t* n_blocks_host, void* stream) {
-  if (!corner_sdf_dev || !block_ids_dev || !workspace_dev || !n_blocks_host) return fail(SDFB_E_INVALID, "null argument");
-  if (res < 2 || block < 1 || block > 64 || !(tau >= 0.f)) return fail(SDFB_E_INVALID, "bad res, block size or tau");
-  size_t need = 0;
-  sdfb_sparse_select_workspace_bytes(res, block, &need);
-  if (workspace_bytes < need) return fail(SDFB_E_INVALID, "workspace holds %zu bytes, %zu needed", workspace_bytes, need);
-  const long long nb = (res - 1 + block - 1) / block, total = nb * nb * nb;
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  uint8_t* ws = static_cast<uint8_t*>(workspace_dev);
-  unsigned char* flags = ws;
-  int* ids_all = reinterpret_cast<int*>(ws + (total + 255) / 256 * 256);
-  int* count_dev = ids_all + total;
-  void* temp = reinterpret_cast<uint8_t*>(count_dev) + 256;
-  CU_TRY(launch_block_select(corner_sdf_dev, static_cast<int>(nb), tau, flags, ids_all, block_ids_dev, count_dev, temp,
-                             block_select_temp_bytes(total), st));
-  int count = 0;
-  CU_TRY(cudaMemcpyAsync(&count, count_dev, sizeof(int), cudaMemcpyDeviceToHost, st));
-  CU_TRY(cudaStreamSynchronize(st));
-  *n_blocks_host = count;
-  return SDFB_OK;
-}
-
-int sdfb_sparse_block_points(int res, int block, const int32_t* block_ids_dev, int64_t n_blocks, float* xyz_dev, void* stream) {
-  if (n_blocks > 0 && (!block_ids_dev || !xyz_dev)) return fail(SDFB_E_INVALID, "null argument");
-  if (res < 2 || block < 1 || block > 64 || n_blocks < 0) return fail(SDFB_E_INVALID, "bad arguments");
-  const int nb = (res - 1 + block - 1) / block;
-  CU_TRY(launch_block_points(res, block, nb, block_ids_dev, n_blocks, xyz_dev, static_cast<cudaStream_t>(stream)));
-  return SDFB_OK;
-}
-
-int sdfb_mc_blocks_workspace_bytes(int block, int64_t n_blocks, size_t* bytes) {
-  if (!bytes || block < 1 || block > 64 || n_blocks < 0) return fail(SDFB_E_INVALID, "bad arguments");
-  const McGeom g = mc_block_geom(2, block, 1, nullptr, n_blocks);
-  *bytes = mc_layout(g.total_nodes, g.total_cells).total;
-  return SDFB_OK;
-}
-
-int sdfb_mc_blocks_count(const float* fields_dev, const int32_t* block_ids_dev, int64_t n_blocks, int res, int block,
-                         void* workspace_dev, size_t workspace_bytes, int64_t* n_triangles_host, void* stream) {
-  if (!n_triangles_host) return fail(SDFB_E_INVALID, "null argument");
-  if (n_blocks == 0) { *n_triangles_host = 0; return SDFB_OK; }
-  if (!fields_dev || !block_ids_dev || !workspace_dev) return fail(SDFB_E_INVALID, "null argument");
-  if (res < 2 || block < 1 || block > 64 || n_blocks < 0) return fail(SDFB_E_INVALID, "bad arguments");
-  const int nb = (res - 1 + block - 1) / block;
-  return mc_count_impl(fields_dev, nullptr, mc_block_geom(res, block, nb, block_ids_dev, n_blocks), workspace_dev, workspace_bytes,
-                       n_triangles_host, static_cast<cudaStream_t>(stream));
-}
-
-int sdfb_mc_blocks_generate(const float* fields_dev, const int32_t* block_ids_dev, int64_t n_blocks, int res, int block,
-                            const void* workspace_dev, float* triangles_dev, int64_t* edge_keys_dev, void* stream) {
-  if (n_blocks == 0) return SDFB_OK;
-  if (!fields_dev || !block_ids_dev || !workspace_dev || !triangles_dev) return fail(SDFB_E_INVALID, "null argument");
-  if (res < 2 || block < 1 || block > 64 || n_blocks < 0) return fail(SDFB_E_INVALID, "bad arguments");
-  const int nb = (res - 1 + block - 1) / block;
-  return mc_generate_impl(fields_dev, mc_block_geom(res, block, nb, block_ids_dev, n_blocks), workspace_dev, triangles_dev,
-                          reinterpret_cast<long long*>(edge_keys_dev), static_cast<cudaStream_t>(stream));
 }
 
 // ---- hierarchical sparse decode (sparse.cu): decode only where the surface can be, hand the dense MC kernels a field that

@@ -298,21 +298,13 @@ cudaError_t launch_mc_weld_count(const long long* keys, long long n_keys, long l
                                  cudaStream_t stream);
 cudaError_t launch_mc_weld_fill(const float* tris, const long long* keys, long long n_keys, long long key_range, const void* workspace,
                                 float* verts, long long* faces, cudaStream_t stream);
-// A field to extract from: a dense [nz][ny][nx] slab whose first plane is plane z0 of the res^3 grid
-// (blocks == nullptr), or a list of blocks of (B+1)^3 nodes each, block id = (bz * nb + by) * nb + bx,
-// stored back to back (the sparse extractor).
+// A field to extract from: a dense [nz][ny][nx] slab whose first plane is plane z0 of the res^3 grid.
 struct McGeom {
   int nz, ny, nx, res, z0;
-  int B, nb;
-  const int* blocks;
   long long total_cells, total_nodes;
 };
 inline McGeom mc_dense_geom(int nz, int ny, int nx, int res, int z0) {
-  return McGeom{nz, ny, nx, res, z0, 0, 0, nullptr, static_cast<long long>(nz - 1) * (ny - 1) * (nx - 1),
-                static_cast<long long>(nz) * ny * nx};
-}
-inline McGeom mc_block_geom(int res, int B, int nb, const int* blocks, long long nblk) {
-  return McGeom{0, 0, 0, res, 0, B, nb, blocks, nblk * B * B * B, nblk * (B + 1) * (B + 1) * (B + 1)};
+  return McGeom{nz, ny, nx, res, z0, static_cast<long long>(nz - 1) * (ny - 1) * (nx - 1), static_cast<long long>(nz) * ny * nx};
 }
 size_t mc_scan_temp_bytes(long long groups);
 cudaError_t launch_mc_count_scan(const unsigned int* bits, const McGeom& g, unsigned int* group_tris, void* temp,
@@ -320,12 +312,6 @@ cudaError_t launch_mc_count_scan(const unsigned int* bits, const McGeom& g, unsi
 // keys (optional, [n_tri * 3]): the grid edge of every emitted vertex, ((z res + y) res + x) * 3 + axis of its lower node
 cudaError_t launch_mc_generate(const float* sdf, const unsigned int* bits, const unsigned int* group_first, const McGeom& g,
                                float* tris, long long* keys, cudaStream_t stream);
-// sparse extractor: block corners, block selection (ascending ids, count on the device), nodes of the selected blocks
-cudaError_t launch_block_corner_points(int res, int B, int nb, float* xyz, cudaStream_t stream);
-size_t block_select_temp_bytes(long long nblocks);
-cudaError_t launch_block_select(const float* corner_sdf, int nb, float tau, unsigned char* flags, int* ids_all, int* ids_out,
-                                int* count_dev, void* temp, size_t temp_bytes, cudaStream_t stream);
-cudaError_t launch_block_points(int res, int B, int nb, const int* blocks, long long nblk, float* xyz, cudaStream_t stream);
 
 // ---- hierarchical sparse decode (sparse.cu) -----------------------------------------------------------------------
 cudaError_t launch_corner_nodes(int res, int B, int nb, unsigned int* idx, cudaStream_t st);

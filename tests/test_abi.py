@@ -70,9 +70,6 @@ def test_workspace_queries_and_validation_of_the_extraction_entry_points(pkg):
     b = C.c_size_t()
     assert lib.sdfb_mc_workspace_bytes(64, 64, 64, C.byref(b)) == 0 and b.value >= 64 ** 3 // 8
     assert lib.sdfb_mc_workspace_bytes(1, 64, 64, C.byref(b)) == -1
-    assert lib.sdfb_sparse_select_workspace_bytes(256, 8, C.byref(b)) == 0 and b.value > 32 ** 3
-    assert lib.sdfb_sparse_select_workspace_bytes(256, 0, C.byref(b)) == -1
-    assert lib.sdfb_mc_blocks_workspace_bytes(8, 1000, C.byref(b)) == 0 and b.value > 1000 * 729 // 8
     n = C.c_int64()
     assert lib.sdfb_mc_count(None, None, 4, 4, 4, None, 0, C.byref(n), None) == -1
     assert lib.sdfb_decoder_vjp_latent(None, None, None, 0, None, None, None, None) == -1

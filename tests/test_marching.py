@@ -184,34 +184,6 @@ def test_cuda_marching_cubes_full_size(pkg, cuda_decoder):
     assert np.array_equal(part.view(np.uint32), want.view(np.uint32))
 
 
-def _sorted_tris(t: np.ndarray) -> np.ndarray:
-    """Triangles as rows of 9 uint32 words, sorted: a canonical form for comparing triangle SETS bit for bit."""
-    w = np.ascontiguousarray(t, dtype=np.float32).reshape(-1, 9).view(np.uint32)
-    return w[np.lexsort(w.T[::-1])]
-
-
-@pytest.mark.gpu
-@pytest.mark.parametrize("res,block", [(64, 4), (97, 8), (128, 5), (256, 8), (256, 4), (512, 8)])
-def test_sparse_extraction_equals_dense(cuda_decoder, res, block):
-    """Decoding only the blocks near the surface gives exactly the dense extraction's triangles
-    (same bits, different order), with a fraction of the queries; ragged last blocks included (97, 128)."""
-    z = oracle.default_latent()
-    dense = cuda_decoder.extract_surface(z, res).cpu().numpy()
-    torch.cuda.synchronize()
-    a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    cuda_decoder.extract_surface_sparse(z, res, block=block, method="blocks")
-    a.record()
-    sparse, st = cuda_decoder.extract_surface_sparse(z, res, block=block, return_stats=True, method="blocks")
-    b.record()
-    b.synchronize()
-    print(f"res {res} block {block}: {st['blocks']}/{st['blocks_total']} blocks, {st['queries']} of {st['dense_queries']} queries "
-          f"({st['dense_queries'] / st['queries']:.1f}x fewer), {sparse.shape[0]} triangles in {a.elapsed_time(b):.2f} ms, L = {st['lipschitz']:.2f}")
-    assert sparse.shape[0] == dense.shape[0]
-    assert np.array_equal(_sorted_tris(sparse.cpu().numpy()), _sorted_tris(dense))
-    if res >= 256:        # the criterion is exact (Lipschitz band), hence conservative: the saving grows with the resolution
-        assert st["queries"] < st["dense_queries"] * (0.5 if res >= 512 else 0.75)
-
-
 @pytest.mark.gpu
 @pytest.mark.parametrize("res,seed,scale", [(64, 0, 1.0), (97, 1, 1.0), (130, 2, 1.0), (256, 0, 1.0), (256, 3, 1.5), (255, 5, 0.5), (512, 0, 1.0)])
 def test_hierarchical_sparse_extraction_equals_dense(cuda_decoder, res, seed, scale):
@@ -272,7 +244,7 @@ def test_hierarchical_sparse_local_slopes_equal_dense(cuda_decoder, res, seed, s
 @pytest.mark.gpu
 def test_indexed_mesh_welding(pkg, cuda_decoder):
     """indexed=True merges vertices by grid edge: the faces index exactly the soup's vertices, a closed surface
-    has Euler characteristic 2, and the sparse extractor welds to the same vertex set."""
+    has Euler characteristic 2, and the sparse extractor welds to the same mesh."""
     f = torch.from_numpy(_sphere(40)).cuda()
     soup = pkg.extract_surface(f)
     verts, faces = pkg.extract_surface(f, indexed=True)
@@ -286,62 +258,45 @@ def test_indexed_mesh_welding(pkg, cuda_decoder):
     assert verts.shape[0] - n_edges + fa.shape[0] == 2                       # a sphere
     z = oracle.default_latent()
     v1, f1 = cuda_decoder.extract_surface(z, 97, indexed=True)
-    v2, f2 = cuda_decoder.extract_surface_sparse(z, 97, block=8, indexed=True, method="blocks")
-    v3, f3 = cuda_decoder.extract_surface_sparse(z, 97, indexed=True)         # two-level path: same soup, same order
-    assert torch.equal(v1, v3) and torch.equal(f1, f3)
-    assert v1.shape == v2.shape and torch.equal(v1, v2)                      # unique() sorts by edge key: identical vertex arrays
-    assert f1.shape == f2.shape
+    v2, f2 = cuda_decoder.extract_surface_sparse(z, 97, indexed=True)         # same soup, same order
+    assert torch.equal(v1, v2) and torch.equal(f1, f2)
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("res,block,thickness_cells", [(96, 8, 1.5), (65, 4, 0.8)])
-def test_block_selection_keeps_a_thin_shell(pkg, res, block, thickness_cells):
-    """A field with a thin feature through the block path of the sparse extractor (corner points -> block selection with the
-    exact Lipschitz threshold -> block nodes -> marching cubes over blocks), fed with an ANALYTIC 1-Lipschitz field instead of
-    the decoder: a spherical shell thinner than a cell or two - two sign changes inside one 8^3 block, none at its corners.
-    The triangle set equals the dense extraction of the same field, and nothing of the shell is lost."""
-    import ctypes as C
-    lib = pkg.load_library()
+@pytest.mark.parametrize("res", [65, 96])
+@pytest.mark.parametrize("width_cells", [0.8, 1.5])
+def test_sparse_extraction_keeps_a_thin_slab(pkg, res, width_cells):
+    """A feature thinner than a block that no block corner sees: a decoder whose field is exactly tanh(|n.x - d| - half),
+    n = (0.5, 0.5, 0.5) - 1-Lipschitz, negative only inside a planar slab `width_cells` cells wide, with d between the planes
+    of level-1 corners.  Layer 0 forms n.x - d and d - n.x (exact bf16 weights), layers 1-7 pass those two channels through
+    with identity weights, the head adds them.  With the bound L = 1 the two-level decode keeps every block and sub-block the
+    slab crosses and the nodes it never decodes inherit the right sign: the soup equals the dense extraction's bit for bit,
+    order included."""
+    from oracle.weights import DEC_LAYER_DIMS
     h = 2.0 / (res - 1)
-    half = 0.5 * thickness_cells * h
-
-    def field(p):                                   # |  |x - c| - r  | - half : 1-Lipschitz, negative inside the shell
-        c = torch.tensor([0.03, -0.02, 0.05], device="cuda")
-        return ((p - c).norm(dim=1) - 0.55).abs() - half
-
-    nb = (res - 1 + block - 1) // block
-    corners = torch.empty(((nb + 1) ** 3, 3), dtype=torch.float32, device="cuda")
-    assert lib.sdfb_sparse_corner_points(res, block, corners.data_ptr(), None) == 0
-    torch.cuda.synchronize()
-    cs = field(corners).contiguous()
-    assert int((cs < 0).sum()) < cs.numel() // 50                                   # the corner lattice hardly sees the shell
-    tau = 1.0 * block * h * (3.0 ** 0.5) / 2.0                                       # Lipschitz constant 1, exact threshold
-    nbytes = C.c_size_t()
-    assert lib.sdfb_sparse_select_workspace_bytes(res, block, C.byref(nbytes)) == 0
-    ws = torch.empty((nbytes.value,), dtype=torch.uint8, device="cuda")
-    ids = torch.empty((nb ** 3,), dtype=torch.int32, device="cuda")
-    nblk = C.c_int64()
-    assert lib.sdfb_sparse_select_blocks(cs.data_ptr(), res, block, C.c_float(tau), ids.data_ptr(), ws.data_ptr(), nbytes.value,
-                                         C.byref(nblk), None) == 0
-    n, per = nblk.value, (block + 1) ** 3
-    assert 0 < n < nb ** 3
-    pts = torch.empty((n * per, 3), dtype=torch.float32, device="cuda")
-    assert lib.sdfb_sparse_block_points(res, block, ids.data_ptr(), n, pts.data_ptr(), None) == 0
-    torch.cuda.synchronize()
-    fields = field(pts).contiguous()
-    assert lib.sdfb_mc_blocks_workspace_bytes(block, n, C.byref(nbytes)) == 0
-    ws2 = torch.empty((nbytes.value,), dtype=torch.uint8, device="cuda")
-    ntri = C.c_int64()
-    assert lib.sdfb_mc_blocks_count(fields.data_ptr(), ids.data_ptr(), n, res, block, ws2.data_ptr(), nbytes.value, C.byref(ntri), None) == 0
-    tris = torch.empty((ntri.value, 3, 3), dtype=torch.float32, device="cuda")
-    assert lib.sdfb_mc_blocks_generate(fields.data_ptr(), ids.data_ptr(), n, res, block, ws2.data_ptr(), tris.data_ptr(), None, None) == 0
-    torch.cuda.synchronize()
-    # dense extraction of the same field on the full grid (the same expression at the same fp32 coordinates)
-    a = torch.from_numpy(oracle.axis_coords(res)).cuda()
-    zz, yy, xx = torch.meshgrid(a, a, a, indexing="ij")
-    dense = field(torch.stack([xx.reshape(-1), yy.reshape(-1), zz.reshape(-1)], dim=1)).reshape(res, res, res).contiguous()
-    ref = pkg.extract_surface(dense)
-    key = lambda t: np.unique(t.cpu().numpy().reshape(-1, 9).view(np.uint32), axis=0)
-    print(f"res {res} block {block}: shell of {thickness_cells} cells, {n} of {nb ** 3} blocks kept, {ntri.value} triangles (dense {ref.shape[0]})")
-    assert ref.shape[0] > 1000 and ntri.value == ref.shape[0]
-    assert np.array_equal(key(tris), key(ref))
+    # n.x at node (i, j, k) is -1.5 + h (i + j + k) / 2: level-1 corners (multiples of 8) lie on the planes n.x = -1.5 + 4h M
+    d = -1.5 + h * (4 * int(0.75 * (res - 1) / 4) + 2.45)
+    half = 0.5 * width_cells * h * np.sqrt(0.75)                                # |n| = sqrt(3) / 2
+    params = [(np.zeros((fout, fin), np.float32), np.zeros(fout, np.float32)) for fin, fout in DEC_LAYER_DIMS]
+    (w0, b0), (w8, b8) = params[0], params[8]
+    w0[0, 256:], b0[0] = 0.5, -d
+    w0[1, 256:], b0[1] = -0.5, d
+    for w, _ in params[1:8]:                                                    # layer 4: columns 0, 1 of [h3 | latent | xyz]
+        w[0, 0] = w[1, 1] = 1.0
+    w8[0, :2], b8[0] = 1.0, -half
+    a = oracle.axis_coords(res).astype(np.float64)[np.minimum(np.arange(0, res + 7, 8), res - 1)]
+    cz, cy, cx = np.meshgrid(a, a, a, indexing="ij")
+    assert not (np.abs(0.5 * (cx + cy + cz) - d) < half).any()                 # no level-1 corner is inside the slab
+    z = np.zeros(256, np.float32)
+    dec = pkg.Decoder(params, device="cuda:0", precision="bf16")
+    try:
+        dense = dec.extract_surface(z, res)
+        sparse, st = dec.extract_surface_sparse(z, res, lipschitz=1.0, return_stats=True)
+    finally:
+        dec.close()
+    print(f"res {res}, slab of {width_cells} cells: {st['queries']} of {st['dense_queries']} queries ({st['corner_queries']} corners, "
+          f"{st['blocks_kept']} blocks, {st['lattice_queries']} lattice nodes, {st['sub_blocks_kept']} sub-blocks, {st['fill_queries']} more), "
+          f"{sparse.shape[0]} triangles")
+    assert dense.shape[0] > 1000
+    assert sparse.shape == dense.shape and torch.equal(sparse, dense)
+    assert st["queries"] < st["dense_queries"]

@@ -33,7 +33,7 @@ def main():
     ap.add_argument("--res", type=int, default=128)
     ap.add_argument("--out", default="shape.obj")
     ap.add_argument("--sampled", action="store_true", help="decode a latent drawn by the DDPM sampler instead of the synthetic one")
-    ap.add_argument("--sparse", action="store_true", help="block-sparse extraction (decode only near the surface)")
+    ap.add_argument("--sparse", action="store_true", help="sparse extraction (decode only near the surface)")
     ap.add_argument("--fit", type=int, default=0, metavar="N", help="refit the shape from N of its own SDF samples (tensor-pipe latent fitting)")
     ap.add_argument("--fit-steps", type=int, default=400)
     args = ap.parse_args()

@@ -31,7 +31,7 @@ for prec in ("fp32", "bf16", "fp16"):
         print("fit", prec, float(loss), float(g.sum()))
 sdf, signs, mw = dec.decode_grid_bits(z, 24, mask=True)
 tri = dec.extract_surface(z, 24)
-tri_s = dec.extract_surface_sparse(z, 33, block=4)
+tri_s = dec.extract_surface_sparse(z, 33)
 print("surface", tuple(tri.shape), tuple(tri_s.shape))
 ddpm = pkg.LatentDDPM(pkg.synthetic.ddpm_params(), device="cuda:0")
 rs = np.random.RandomState(0)
