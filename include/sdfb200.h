@@ -227,7 +227,8 @@ int sdfb_ddpm_destroy(sdfb_ddpm* ddpm);
  * linear-beta schedule with the x0-clipped posterior-mean update.
  * steps < 1000 TRUNCATES that schedule (it is not respaced: the coefficients stay those of the 1000-step
  * chain), which is what the short parity tests and the profilers want; samples of the trained distribution
- * need steps = 1000.  1 <= steps <= 1000, anything else is SDFB_E_INVALID. */
+ * need steps = 1000, or a respaced schedule (sdfb_ddpm_sample_ddim below).  1 <= steps <= 1000, anything else
+ * is SDFB_E_INVALID. */
 int sdfb_ddpm_sample(sdfb_ddpm* ddpm, float* x_dev, const float* noise_dev, int n, int steps,
                      int precision, void* stream);
 /* one denoiser evaluation eps_hat(x, t) -> eps_dev [n][256] */
@@ -247,6 +248,36 @@ int sdfb_ddpm_sample_philox(sdfb_ddpm* ddpm, float* x_dev, uint64_t seed, int64_
                             int gen_xT, int precision, void* stream);
 int sdfb_ddpm_sample_philox_host(sdfb_ddpm* ddpm, float* x_host, uint64_t seed, int64_t first_latent, int n, int steps,
                                  int gen_xT, int precision);
+/* ---- respaced schedules: DDIM sampling and deterministic DDIM inversion ----
+ * abar_t is the 1000-step linear-beta schedule above (fp64).  S steps visit tau_i = floor(i 1000 / S), i = 0 .. S-1
+ * (S = 1000: every t).  Each step evaluates eps_hat at its timestep and applies
+ *   x0 = clamp(sra x - srm1 eps_hat, -clamp, clamp);  x <- c1 x0 + c2 x [+ c3 eps_hat] [+ sigma z]
+ * (products and sums rounded one by one in that order; the c3 term only when c3 != 0, the noise term only when sigma != 0).
+ * Sampling, i = S-1 .. 0 from x at tau_i, with a = abar_{tau_i}, a' = abar_{tau_{i-1}} (1 for i = 0):
+ *   sigma = eta sqrt((1 - a') / (1 - a)) sqrt(1 - a / a'),  c2 = sqrt(max(0, 1 - a' - sigma^2)) / sqrt(1 - a),
+ *   c1 = sqrt(a') - c2 sqrt(a), c3 = 0, clamp = 1; eta = 1 at S = 1000 is the DDPM posterior of sdfb_ddpm_sample,
+ *   eta = 0 is deterministic.  The last step (i = 0) has c1 = 1, c2 = sigma = 0.
+ * Inversion, i = 0 .. S-1 from a clean x0 to x at tau_{S-1}, with a = abar_{tau_{i-1}} (1 for i = 0), a' = abar_{tau_i}:
+ *   sra, srm1 of a, c1 = sqrt(a'), c2 = 0, c3 = sqrt(1 - a'), sigma = 0, clamp = +inf (x0 is not clamped).
+ *
+ * sdfb_ddim_schedule: host only, no device.  timesteps_host [steps] and coef_host [steps][8] = (sra, srm1, c1, c2, c3, sigma,
+ * clamp, 0) receive the rows in execution order.  1 <= steps <= 1000 and 0 <= eta <= 1 (finite), else SDFB_E_INVALID
+ * (inverse != 0: eta is checked but unused).  The entry points below run exactly these rows.
+ *
+ * Noise.  Explicit: noise_dev [steps][n][256], noise[i] is consumed at the step from tau_i (noise[0] is never read); it may be
+ * NULL when eta = 0 (a NULL stream with eta > 0 is SDFB_E_INVALID).  Seeded: the Philox counter's step field is tau_i, so
+ * DDIM at S = 1000, eta = 1 draws the numbers of sdfb_ddpm_sample_philox; gen_xT != 0 takes x_T from row t = 1000 of the
+ * stream whatever S is (the same seed starts DDIM-S and the full 1000-step chain from the same x_T).  A step with sigma = 0
+ * (every step at eta = 0) reads and generates no noise.
+ * precision, the watchdog, the status mirror and sdfb_ddpm_last_kernel_ms behave as for sdfb_ddpm_sample; bf16 / fp16 run
+ * all S steps in one launch of the same fused kernel.  x_dev holds x_T on entry and x_0 on return (invert: x0 on entry,
+ * x at tau_{S-1} on return, in place). */
+int sdfb_ddim_schedule(int steps, float eta, int inverse, int32_t* timesteps_host, float* coef_host);
+int sdfb_ddpm_sample_ddim(sdfb_ddpm* ddpm, float* x_dev, const float* noise_dev, int n, int steps, float eta, int precision,
+                          void* stream);
+int sdfb_ddpm_sample_ddim_philox(sdfb_ddpm* ddpm, float* x_dev, uint64_t seed, int64_t first_latent, int n, int steps, float eta,
+                                 int gen_xT, int precision, void* stream);
+int sdfb_ddpm_invert_ddim(sdfb_ddpm* ddpm, float* x_dev, int n, int steps, int precision, void* stream);
 /* The stream itself: normals of steps [t0, t1) for latents [first_latent, first_latent + n)
  * -> out_dev [(t1-t0)][n][256]. */
 int sdfb_philox_normal(uint64_t seed, int64_t first_latent, int n, int t0, int t1, float* out_dev, void* stream);

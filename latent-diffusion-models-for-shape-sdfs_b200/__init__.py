@@ -15,6 +15,7 @@ The directory name contains hyphens, so import it with
 """
 from ._lib import PRECISIONS, SdfbError, load as load_library  # noqa: F401
 from .api import (Decoder, LatentDDPM, DDPMTrainer, DecoderTrainer, Comm, decode_grid, sample_latents, grid_points, sign_change_mask, philox_normal,  # noqa: F401
+                  ddim_schedule,
                   extract_surface, weld, unpack_mask_blocks, DDPM_LATENT_SCALE)
 from .sharding import (slab_range, batch_range, decode_grid_sharded, decode_batch_sharded, sample_latents_sharded,  # noqa: F401
                        fit_latents_sharded)

@@ -66,6 +66,10 @@ SIGNATURES = {
     "sdfb_ddpm_sample_philox": (_i, [_vp, _vp, C.c_uint64, _i64, _i, _i, _i, _i, _vp]),
     "sdfb_ddpm_sample_philox_host": (_i, [_vp, _vp, C.c_uint64, _i64, _i, _i, _i, _i]),
     "sdfb_philox_normal": (_i, [C.c_uint64, _i64, _i, _i, _i, _vp, _vp]),
+    "sdfb_ddim_schedule": (_i, [_i, C.c_float, _i, _vp, _vp]),
+    "sdfb_ddpm_sample_ddim": (_i, [_vp, _vp, _vp, _i, _i, C.c_float, _i, _vp]),
+    "sdfb_ddpm_sample_ddim_philox": (_i, [_vp, _vp, C.c_uint64, _i64, _i, _i, C.c_float, _i, _i, _vp]),
+    "sdfb_ddpm_invert_ddim": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "sdfb_ddpm_trainer_create": (_i, [_vp, _sz, _i, _i, C.POINTER(_vp)]),
     "sdfb_ddpm_trainer_destroy": (_i, [_vp]),
     "sdfb_ddpm_trainer_step": (_i, [_vp, _vp, _vp, _vp, _i, C.c_float, C.c_float, C.c_float, C.c_float, _i, _vp, _vp, _vp]),

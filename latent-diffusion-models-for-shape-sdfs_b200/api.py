@@ -480,6 +480,48 @@ class LatentDDPM:
             self.last_kernel_ms()       # waits for the persistent kernel and raises if its watchdog tripped
         return x
 
+    def sample_latents_ddim(self, n: int, steps: int = 50, eta: float = 0.0, x_T=None, noise=None, seed: int = 0,
+                            precision: str | None = None, first_latent: int = 0) -> torch.Tensor:
+        """x_0 [n,256] by DDIM (Song et al. 2021) on ``steps`` respaced timesteps tau_i = floor(i 1000 / steps) of the
+        1000-step chain.  ``eta`` = 0 is deterministic given x_T; ``eta`` = 1 at ``steps`` = 1000 is the DDPM chain of
+        ``sample_latents``.  ``noise`` [steps,n,256] (with ``x_T``) is an explicit stream, noise[i] consumed at the step
+        from tau_i; it is not needed at ``eta`` = 0.  Without it the stream is generated in the kernel from ``seed``
+        (Philox step field tau_i; x_T, when not given, from row 1000, so the same seed starts every step count from the
+        same x_T).  ``first_latent`` as in ``sample_latents``.  The rows run are those of ``ddim_schedule``."""
+        prec = _prec(precision or self.precision)
+        if n <= 0:
+            raise ValueError("n must be positive")
+        if noise is None and x_T is None:
+            x = torch.empty((n, LATENT), dtype=torch.float32, device=self.device)
+        elif x_T is None:
+            raise ValueError("an explicit noise stream needs an explicit x_T")
+        else:
+            x = _as_dev_f32(x_T, self.device, (n, LATENT)).clone()
+        st = _stream_ptr(self.device.index)
+        if noise is None:
+            check(self._lib.sdfb_ddpm_sample_ddim_philox(self._h, x.data_ptr(), int(seed), int(first_latent), n, int(steps),
+                                                         float(eta), 1 if x_T is None else 0, prec, st))
+        else:
+            nz = _as_dev_f32(noise, self.device, (int(steps), n, LATENT))
+            check(self._lib.sdfb_ddpm_sample_ddim(self._h, x.data_ptr(), nz.data_ptr(), n, int(steps), float(eta), prec, st))
+        if prec != _lib.PREC_FP32:
+            self.last_kernel_ms()       # waits for the persistent kernel and raises if its watchdog tripped
+        return x
+
+    def invert_latents_ddim(self, x0, steps: int = 50, precision: str | None = None) -> torch.Tensor:
+        """Deterministic DDIM inversion: the x_T [n,256] (at timestep tau_{steps-1}) from which ``sample_latents_ddim`` with
+        the same ``steps`` and ``eta`` = 0 returns to ``x0`` [n,256] (up to the denoiser's sensitivity to its input and
+        rounding).  ``x0`` lives in the DDPM's space: a decoder latent (e.g. from ``Decoder.fit_latent``) must be divided by
+        ``DDPM_LATENT_SCALE`` first.  x0 is not clipped to [-1, 1] on the way."""
+        prec = _prec(precision or self.precision)
+        x = _as_dev_f32(x0, self.device).clone()
+        if x.ndim != 2 or x.shape[1] != LATENT or x.shape[0] == 0:
+            raise ValueError("x0 must be [n,256] with n > 0")
+        check(self._lib.sdfb_ddpm_invert_ddim(self._h, x.data_ptr(), x.shape[0], int(steps), prec, _stream_ptr(self.device.index)))
+        if prec != _lib.PREC_FP32:
+            self.last_kernel_ms()
+        return x
+
     def check(self) -> None:
         """Waits for the current stream; raises SdfbError if the fused sampler's watchdog tripped."""
         check(self._lib.sdfb_ddpm_check(self._h, _stream_ptr(self.device.index)))
@@ -728,6 +770,16 @@ def decode_grid(decoder: Decoder, z, res: int, **kw):
 
 def sample_latents(ddpm: LatentDDPM, n: int, **kw):
     return ddpm.sample_latents(n, **kw)
+
+
+def ddim_schedule(steps: int, eta: float, inverse: bool = False):
+    """The rows a respaced call runs, in execution order (``sdfb_ddim_schedule``; no device needed):
+    timesteps int32 [steps] and coefficients float32 [steps, 8] = (sra, srm1, c1, c2, c3, sigma, clamp, 0)."""
+    lib = _lib.load()
+    ts = np.zeros(int(steps) if int(steps) > 0 else 0, np.int32)
+    coef = np.zeros((ts.size, 8), np.float32)
+    check(lib.sdfb_ddim_schedule(int(steps), float(eta), 1 if inverse else 0, ts.ctypes.data, coef.ctypes.data))
+    return ts, coef
 
 
 def philox_normal(seed: int, n: int, t0: int, t1: int, device="cuda:0", first_latent: int = 0) -> torch.Tensor:

@@ -1,11 +1,13 @@
 // C ABI of libsdfb200.so (declared in include/sdfb200.h): contexts, weight packing,
 // argument validation and kernel launches.  No reference interface exists to mirror
 // (/root/reference/README.md:1 is a title); the surface follows SURVEY.md section 8(b).
+#include <algorithm>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <new>
 #include <vector>
 
@@ -230,7 +232,7 @@ struct sdfb_ddpm {
   float* params = nullptr;
   long long woff[5], boff[5];
   float* tb0 = nullptr;          // [1000][1024]: b0 + W0[:, 256:] temb(t)
-  std::vector<float> sra, srm1, c1, c2, sigma;
+  std::vector<DdpmStep> ddpm_rows;            // the 1000-step DDPM chain in execution order (t = 999 .. 0), fp32 coefficients
   int ws_n = 0;
   float *h0 = nullptr, *h1 = nullptr, *eps = nullptr;
   void* dstage = nullptr; size_t dstage_bytes = 0;
@@ -238,7 +240,8 @@ struct sdfb_ddpm {
   // tensor-core path (ddpm_step.cu)
   uint8_t* wpack[2] = {nullptr, nullptr};     // [0] bf16, [1] fp16: kDdpmWRows rows of 128 B
   float* bias_dev = nullptr;                  // [3][1024] + [256]
-  float* coef_dev = nullptr;                  // [1000][8]
+  DdpmStep* ddpm_rows_dev = nullptr;          // ddpm_rows on the device: a truncated chain of `steps` is its last `steps` rows
+  DdpmStep* call_rows_dev = nullptr;          // [1000]: the rows of a respaced (DDIM) call, written on the caller's stream
   DdpmLane lane[2];                           // workspaces of the (at most two) concurrent launches of a call
   cudaStream_t st_b = nullptr; cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   unsigned int* status = nullptr;
@@ -1402,21 +1405,26 @@ int sdfb_ddpm_create(const float* params_host, size_t n_floats, int device, sdfb
   } while (0)
   CU_TRY_D(cudaMalloc(&d->params, n_floats * sizeof(float)));
   CU_TRY_D(cudaMemcpy(d->params, params_host, n_floats * sizeof(float), cudaMemcpyHostToDevice));
-  // A5: schedule in fp64, cast to fp32 (oracle/ddpm.py ddpm_schedule)
+  // A5: schedule in fp64, cast to fp32 (oracle/ddpm.py ddpm_schedule), as the DDPM table: t = 999 .. 0, noise plane t,
+  // no eps term, clamp bound 1
   {
     const int T = kDdpmT;
-    d->sra.resize(T); d->srm1.resize(T); d->c1.resize(T); d->c2.resize(T); d->sigma.resize(T);
+    d->ddpm_rows.assign(T, DdpmStep{});
     double abar = 1.0, abar_prev = 1.0;
     for (int t = 0; t < T; ++t) {
       const double beta = 1e-4 + (0.02 - 1e-4) * static_cast<double>(t) / (T - 1);
       const double alpha = 1.0 - beta;
       abar_prev = abar;
       abar = abar * alpha;
-      d->sra[t] = static_cast<float>(1.0 / std::sqrt(abar));
-      d->srm1[t] = static_cast<float>(std::sqrt(1.0 / abar - 1.0));
-      d->c1[t] = static_cast<float>(beta * std::sqrt(abar_prev) / (1.0 - abar));
-      d->c2[t] = static_cast<float>((1.0 - abar_prev) * std::sqrt(alpha) / (1.0 - abar));
-      d->sigma[t] = t == 0 ? 0.f : static_cast<float>(std::sqrt(beta * (1.0 - abar_prev) / (1.0 - abar)));
+      DdpmStep& r = d->ddpm_rows[T - 1 - t];
+      r.coef[0] = static_cast<float>(1.0 / std::sqrt(abar));
+      r.coef[1] = static_cast<float>(std::sqrt(1.0 / abar - 1.0));
+      r.coef[2] = static_cast<float>(beta * std::sqrt(abar_prev) / (1.0 - abar));
+      r.coef[3] = static_cast<float>((1.0 - abar_prev) * std::sqrt(alpha) / (1.0 - abar));
+      r.coef[5] = t == 0 ? 0.f : static_cast<float>(std::sqrt(beta * (1.0 - abar_prev) / (1.0 - abar)));
+      r.coef[6] = 1.f;
+      r.t = t;
+      r.plane = t;
     }
   }
   // time-embedding half of layer 0 folded into a per-step bias table
@@ -1453,13 +1461,9 @@ int sdfb_ddpm_create(const float* params_host, size_t n_floats, int device, sdfb
     std::memcpy(hb.data() + 3 * kDdpmHid, params_host + d->boff[4], kDdpmLatent * sizeof(float));
     CU_TRY_D(cudaMalloc(&d->bias_dev, hb.size() * sizeof(float)));
     CU_TRY_D(cudaMemcpy(d->bias_dev, hb.data(), hb.size() * sizeof(float), cudaMemcpyHostToDevice));
-    std::vector<float> hc(static_cast<size_t>(kDdpmT) * 8, 0.f);
-    for (int t = 0; t < kDdpmT; ++t) {
-      hc[t * 8 + 0] = d->sra[t]; hc[t * 8 + 1] = d->srm1[t]; hc[t * 8 + 2] = d->c1[t]; hc[t * 8 + 3] = d->c2[t];
-      hc[t * 8 + 4] = d->sigma[t];
-    }
-    CU_TRY_D(cudaMalloc(&d->coef_dev, hc.size() * sizeof(float)));
-    CU_TRY_D(cudaMemcpy(d->coef_dev, hc.data(), hc.size() * sizeof(float), cudaMemcpyHostToDevice));
+    CU_TRY_D(cudaMalloc(&d->ddpm_rows_dev, kDdpmT * sizeof(DdpmStep)));
+    CU_TRY_D(cudaMemcpy(d->ddpm_rows_dev, d->ddpm_rows.data(), kDdpmT * sizeof(DdpmStep), cudaMemcpyHostToDevice));
+    CU_TRY_D(cudaMalloc(&d->call_rows_dev, kDdpmT * sizeof(DdpmStep)));
   }
   CU_TRY_D(cudaMalloc(&d->status, sizeof(unsigned int)));
   CU_TRY_D(cudaMemset(d->status, 0, sizeof(unsigned int)));
@@ -1483,7 +1487,7 @@ int sdfb_ddpm_destroy(sdfb_ddpm* d) {
   DeviceGuard g(d->device);
   cudaDeviceSynchronize();
   cudaFree(d->params); cudaFree(d->tb0); cudaFree(d->h0); cudaFree(d->h1); cudaFree(d->eps); cudaFree(d->dstage);
-  cudaFree(d->wpack[0]); cudaFree(d->wpack[1]); cudaFree(d->bias_dev); cudaFree(d->coef_dev);
+  cudaFree(d->wpack[0]); cudaFree(d->wpack[1]); cudaFree(d->bias_dev); cudaFree(d->ddpm_rows_dev); cudaFree(d->call_rows_dev);
   for (DdpmLane& L : d->lane) { cudaFree(L.act); cudaFree(L.counter); }
   if (d->st_b) cudaStreamDestroy(d->st_b);
   if (d->ev_fork) cudaEventDestroy(d->ev_fork);
@@ -1522,11 +1526,26 @@ static int denoise_fp32(sdfb_ddpm* d, const float* x, int t, int n, float* eps, 
   return SDFB_OK;
 }
 
-// Tensor-core path: `steps` fused denoise+update steps t = t_first, t_first-1, ... in ONE cooperative
-// launch (eps_out != nullptr: a single denoiser evaluation, no update).
-// One launch of the fused sampler over latents [0, n) of (x, noise) with workspace `lane`.  `noise_batch` is the
-// latent count of the noise tensor's step stride (> n when this launch covers a share of a batch); bn_force = 0: auto.
-static int ddpm_tc_lane(sdfb_ddpm* d, int lane, float* x, const float* noise, long long noise_batch, int n, int steps, int t_first,
+// FFMA path: the schedule rows `rows` (host memory, execution order), one denoiser evaluation and one update each; the
+// noise of a row is plane `plane` of the stream and is read only when its sigma != 0.
+static int sample_fp32(sdfb_ddpm* d, float* x, const float* noise, int n, const DdpmStep* rows, int steps, cudaStream_t st) {
+  int rc = ddpm_ws(d, n);
+  if (rc) return rc;
+  const long long cnt = static_cast<long long>(n) * kDdpmLatent;
+  for (int s = 0; s < steps; ++s) {
+    const DdpmStep& r = rows[s];
+    rc = denoise_fp32(d, x, r.t, n, d->eps, st);
+    if (rc) return rc;
+    CU_TRY(launch_ddpm_update(x, d->eps, r.coef[5] != 0.f ? noise + static_cast<size_t>(r.plane) * cnt : nullptr, cnt, r.coef, st));
+  }
+  return SDFB_OK;
+}
+
+// One launch of the fused sampler over latents [0, n) of (x, noise) with workspace `lane`: the `steps` schedule rows
+// `rows` (device memory, execution order), or (eps_out != nullptr) a single denoiser evaluation at rows[0].t.  The
+// explicit noise stream has `steps` planes; `noise_batch` is the latent count of its plane stride (> n when this launch
+// covers a share of a batch); bn_force = 0: auto.
+static int ddpm_tc_lane(sdfb_ddpm* d, int lane, float* x, const float* noise, long long noise_batch, int n, const DdpmStep* rows, int steps,
                         float* eps_out, bool fp16, cudaStream_t st, bool philox, unsigned long long seed, unsigned int first_latent,
                         int bn_force, bool time_it) {
   DdpmLane& L = d->lane[lane];
@@ -1551,10 +1570,10 @@ static int ddpm_tc_lane(sdfb_ddpm* d, int lane, float* x, const float* noise, lo
     if (v == 64 || v == 128 || v == 256) bn_h = v;
   }
   DdpmParams p{};
-  p.tb0 = d->tb0; p.bias = d->bias_dev; p.coef = d->coef_dev;
+  p.tb0 = d->tb0; p.bias = d->bias_dev; p.sched = rows;
   p.eps_mode = eps_out != nullptr ? 1 : 0;
   p.philox = philox ? 1 : 0; p.seed = seed; p.first_latent = first_latent;
-  p.n = n; p.pair_m_tiles = m_pairs; p.steps = steps; p.t_first = t_first;
+  p.n = n; p.pair_m_tiles = m_pairs; p.steps = steps;
   p.bn_h = bn_h;
   p.nstages = bn_h == 256 ? 5 : (bn_h == 128 ? 6 : 8);   // 5 x 32 KiB, 6 x 24 KiB or 8 x 20 KiB of operand ring + 64 KiB of epilogue staging
   // the four pair tiles of a latent group as ONE cluster of 8 CTAs (cluster-scope group barrier) when every pair has
@@ -1598,12 +1617,12 @@ static int ddpm_tc_lane(sdfb_ddpm* d, int lane, float* x, const float* noise, lo
     const unsigned x_box[2] = {32, 128};
     CU_TRY(make_tensor_map(maps.x, eps_out != nullptr ? eps_out : x, 4, 2, x_dims, x_str, x_box, true));
     if (noise != nullptr && eps_out == nullptr) {
-      const unsigned long long n_dims[3] = {kDdpmLatent, static_cast<unsigned long long>(n), static_cast<unsigned long long>(t_first + 1)};
+      const unsigned long long n_dims[3] = {kDdpmLatent, static_cast<unsigned long long>(n), static_cast<unsigned long long>(steps)};
       const unsigned long long n_str[2] = {kDdpmLatent * 4ull, static_cast<unsigned long long>(noise_batch) * kDdpmLatent * 4ull};
       const unsigned n_box[3] = {32, 128, 1};
       CU_TRY(make_tensor_map(maps.nz, noise, 4, 3, n_dims, n_str, n_box, true));
     } else {
-      std::memcpy(maps.nz, maps.x, 128);   // never dereferenced (t_first == 0 or eps_mode)
+      std::memcpy(maps.nz, maps.x, 128);   // never dereferenced (eps_mode, seeded, or sigma = 0 in every row)
     }
   }
   CU_TRY(launch_ddpm_split(x, n, n_pad, L.act, fp16, st));
@@ -1614,11 +1633,11 @@ static int ddpm_tc_lane(sdfb_ddpm* d, int lane, float* x, const float* noise, lo
   return SDFB_OK;
 }
 
-// Tensor-core path: `steps` fused denoise+update steps t = t_first, t_first-1, ... in ONE cooperative launch
+// Tensor-core path: the `steps` schedule rows `rows` (device memory; fused denoise + update steps) in ONE cooperative launch
 // (eps_out != nullptr: a single denoiser evaluation, no update) - or in TWO concurrent launches when the batch has
 // one to three latent groups more than fit the 8-CTA-cluster mode: the groups that fit run in that mode (they have no
 // dependency outside their cluster), the rest as plain CTA pairs on the SMs that are left, on a second stream.
-static int ddpm_tc(sdfb_ddpm* d, float* x, const float* noise, int n, int steps, int t_first, float* eps_out,
+static int ddpm_tc(sdfb_ddpm* d, float* x, const float* noise, int n, const DdpmStep* rows, int steps, float* eps_out,
                    bool fp16, cudaStream_t st, bool philox = false, unsigned long long seed = 0, unsigned int first_latent = 0) {
   const int m_pairs = (n + 255) / 256;
   const int f = fp16 ? 1 : 0;
@@ -1634,7 +1653,7 @@ static int ddpm_tc(sdfb_ddpm* d, float* x, const float* noise, int n, int steps,
     if (2 * groups_b * (kDdpmHid / bn_b) > d->num_sms - 8 * c8) split = false;    // the rest must be resident beside the clusters
   }
   if (!split) {
-    int rc = ddpm_tc_lane(d, 0, x, noise, n, n, steps, t_first, eps_out, fp16, st, philox, seed, first_latent, 0, true);
+    int rc = ddpm_tc_lane(d, 0, x, noise, n, n, rows, steps, eps_out, fp16, st, philox, seed, first_latent, 0, true);
     if (rc) return rc;
     CU_TRY(cudaEventRecord(d->ev1, st));
     d->timed = true;
@@ -1649,10 +1668,11 @@ static int ddpm_tc(sdfb_ddpm* d, float* x, const float* noise, int n, int steps,
   CU_TRY(cudaEventRecord(d->ev0, st));
   CU_TRY(cudaEventRecord(d->ev_fork, st));
   CU_TRY(cudaStreamWaitEvent(d->st_b, d->ev_fork, 0));
-  int rc = ddpm_tc_lane(d, 0, x, noise, n, n_a, steps, t_first, nullptr, fp16, st, philox, seed, first_latent, 256, false);
+  // (both launches read the same schedule rows)
+  int rc = ddpm_tc_lane(d, 0, x, noise, n, n_a, rows, steps, nullptr, fp16, st, philox, seed, first_latent, 256, false);
   if (rc) return rc;
   rc = ddpm_tc_lane(d, 1, x + static_cast<size_t>(n_a) * kDdpmLatent, noise ? noise + static_cast<size_t>(n_a) * kDdpmLatent : nullptr, n,
-                    n_b, steps, t_first, nullptr, fp16, d->st_b, philox, seed, first_latent + static_cast<unsigned int>(n_a), bn_b, false);
+                    n_b, rows, steps, nullptr, fp16, d->st_b, philox, seed, first_latent + static_cast<unsigned int>(n_a), bn_b, false);
   if (rc) return rc;
   CU_TRY(cudaEventRecord(d->ev_join, d->st_b));
   CU_TRY(cudaStreamWaitEvent(st, d->ev_join, 0));
@@ -1744,7 +1764,7 @@ int sdfb_ddpm_denoise(sdfb_ddpm* d, const float* x_dev, int t, int n, float* eps
   DeviceGuard g(d->device);
   if (int prc = ddpm_pending_status(d)) return prc;
   if (precision != SDFB_PREC_FP32)
-    return ddpm_tc(d, const_cast<float*>(x_dev), nullptr, n, 1, t, eps_dev, precision == SDFB_PREC_FP16,
+    return ddpm_tc(d, const_cast<float*>(x_dev), nullptr, n, d->ddpm_rows_dev + (kDdpmT - 1 - t), 1, eps_dev, precision == SDFB_PREC_FP16,
                    static_cast<cudaStream_t>(stream));
   int rc = ddpm_ws(d, n);
   if (rc) return rc;
@@ -1762,17 +1782,8 @@ int sdfb_ddpm_sample(sdfb_ddpm* d, float* x_dev, const float* noise_dev, int n, 
   if (int prc = ddpm_pending_status(d)) return prc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (precision != SDFB_PREC_FP32)
-    return ddpm_tc(d, x_dev, noise_dev, n, steps, steps - 1, nullptr, precision == SDFB_PREC_FP16, st);
-  int rc = ddpm_ws(d, n);
-  if (rc) return rc;
-  const long long cnt = static_cast<long long>(n) * kDdpmLatent;
-  for (int t = steps - 1; t >= 0; --t) {
-    rc = denoise_fp32(d, x_dev, t, n, d->eps, st);
-    if (rc) return rc;
-    CU_TRY(launch_ddpm_update(x_dev, d->eps, t > 0 ? noise_dev + static_cast<size_t>(t) * cnt : nullptr, cnt,
-                              d->sra[t], d->srm1[t], d->c1[t], d->c2[t], d->sigma[t], st));
-  }
-  return SDFB_OK;
+    return ddpm_tc(d, x_dev, noise_dev, n, d->ddpm_rows_dev + (kDdpmT - steps), steps, nullptr, precision == SDFB_PREC_FP16, st);
+  return sample_fp32(d, x_dev, noise_dev, n, d->ddpm_rows.data() + (kDdpmT - steps), steps, st);
 }
 
 int sdfb_philox_normal(uint64_t seed, int64_t first_latent, int n, int t0, int t1, float* out_dev, void* stream) {
@@ -1796,7 +1807,7 @@ int sdfb_ddpm_sample_philox(sdfb_ddpm* d, float* x_dev, uint64_t seed, int64_t f
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   if (gen_xT) CU_TRY(launch_philox_normal(seed, f0, n, steps, steps + 1, x_dev, st));  // x_T = row t = steps of the stream
   if (precision != SDFB_PREC_FP32)
-    return ddpm_tc(d, x_dev, nullptr, n, steps, steps - 1, nullptr, precision == SDFB_PREC_FP16, st, true, seed, f0);
+    return ddpm_tc(d, x_dev, nullptr, n, d->ddpm_rows_dev + (kDdpmT - steps), steps, nullptr, precision == SDFB_PREC_FP16, st, true, seed, f0);
   // fp32 path: materialise the same stream (bit for bit the in-kernel one) and run the FFMA sampler on it
   const size_t cnt = static_cast<size_t>(n) * kDdpmLatent;
   int rc = ensure_stage(nullptr, nullptr, &d->nstage, &d->nstage_bytes, 0, static_cast<size_t>(steps) * cnt * sizeof(float));
@@ -1842,6 +1853,127 @@ int sdfb_ddpm_sample_host(sdfb_ddpm* d, float* x_host, const float* noise_host, 
   CU_TRY(cudaMemcpyAsync(x_host, x, cnt * sizeof(float), cudaMemcpyDeviceToHost, 0));
   CU_TRY(cudaStreamSynchronize(0));
   return precision == SDFB_PREC_FP32 ? SDFB_OK : ddpm_status(d);
+}
+
+// ---- respaced (DDIM) schedules ----
+
+// The rows of sdfb_ddim_schedule as the sampler's table: the timestep selects the time-embedding bias and the Philox
+// counter, the plane is the step index i (noise[i] is consumed at the step from tau_i).
+static int ddim_rows(int steps, float eta, int inverse, std::vector<DdpmStep>& rows) {
+  std::vector<int32_t> ts(static_cast<size_t>(steps));
+  std::vector<float> coef(static_cast<size_t>(steps) * 8);
+  int rc = sdfb_ddim_schedule(steps, eta, inverse, ts.data(), coef.data());
+  if (rc) return rc;
+  rows.assign(static_cast<size_t>(steps), DdpmStep{});
+  for (int k = 0; k < steps; ++k) {
+    std::memcpy(rows[k].coef, coef.data() + static_cast<size_t>(k) * 8, 8 * sizeof(float));
+    rows[k].t = ts[k];
+    rows[k].plane = inverse ? k : steps - 1 - k;
+  }
+  return SDFB_OK;
+}
+
+int sdfb_ddim_schedule(int steps, float eta, int inverse, int32_t* timesteps_host, float* coef_host) {
+  if (!timesteps_host || !coef_host) return fail(SDFB_E_INVALID, "null argument");
+  if (steps < 1 || steps > kDdpmT) return fail(SDFB_E_INVALID, "steps must be in [1, %d], got %d", kDdpmT, steps);
+  if (!(eta >= 0.f && eta <= 1.f)) return fail(SDFB_E_INVALID, "eta must be a finite value in [0, 1]");
+  // abar of the 1000-step linear-beta chain in fp64, with beta = numpy.linspace(1e-4, 0.02, 1000) to the last bit
+  const int T = kDdpmT;
+  std::vector<double> abar(T);
+  {
+    const double start = 1e-4, stop = 0.02, step = (stop - start) / (T - 1);
+    double a = 1.0;
+    for (int t = 0; t < T; ++t) {
+      const double beta = t == T - 1 ? stop : static_cast<double>(t) * step + start;
+      a = a * (1.0 - beta);
+      abar[t] = a;
+    }
+  }
+  auto tau = [&](int i) { return static_cast<int>(static_cast<long long>(i) * T / steps); };
+  const double e = static_cast<double>(eta);
+  const float inf = std::numeric_limits<float>::infinity();
+  for (int k = 0; k < steps; ++k) {
+    const int i = inverse ? k : steps - 1 - k;              // rows in execution order
+    float* c = coef_host + static_cast<size_t>(k) * 8;
+    timesteps_host[k] = tau(i);
+    if (inverse) {
+      // from x at tau_{i-1} (x0 itself for i = 0) to x at tau_i, with eps evaluated at tau_i; x0 is not clamped
+      const double cur = i > 0 ? abar[tau(i - 1)] : 1.0, next = abar[tau(i)];
+      const double v[8] = {1.0 / std::sqrt(cur), std::sqrt(1.0 / cur - 1.0), std::sqrt(next), 0.0, std::sqrt(1.0 - next), 0.0, 0.0, 0.0};
+      for (int j = 0; j < 8; ++j) c[j] = static_cast<float>(v[j]);
+      c[6] = inf;
+    } else {
+      const double ab = abar[tau(i)], abp = i > 0 ? abar[tau(i - 1)] : 1.0;
+      const double sigma = e * std::sqrt((1.0 - abp) / (1.0 - ab)) * std::sqrt(1.0 - ab / abp);
+      const double c2 = std::sqrt(std::max(0.0, 1.0 - abp - sigma * sigma)) / std::sqrt(1.0 - ab);
+      const double c1 = std::sqrt(abp) - c2 * std::sqrt(ab);
+      const double v[8] = {1.0 / std::sqrt(ab), std::sqrt(1.0 / ab - 1.0), c1, c2, 0.0, sigma, 1.0, 0.0};
+      for (int j = 0; j < 8; ++j) c[j] = static_cast<float>(v[j]);
+    }
+  }
+  return SDFB_OK;
+}
+
+// The checks every respaced entry point shares; on success the schedule rows are in `rows`.
+static int ddim_prepare(sdfb_ddpm* d, const float* x_dev, int n, int steps, float eta, int inverse, int precision,
+                        std::vector<DdpmStep>& rows) {
+  if (!d || !x_dev) return fail(SDFB_E_INVALID, "null argument");
+  if (n <= 0) return fail(SDFB_E_INVALID, "bad n");
+  if (precision != SDFB_PREC_FP32 && precision != SDFB_PREC_BF16 && precision != SDFB_PREC_FP16)
+    return fail(SDFB_E_INVALID, "unknown precision %d", precision);
+  return ddim_rows(steps, eta, inverse, rows);
+}
+
+// Runs the rows: the fused kernel reads them from the context's call table, written on the caller's stream and so ordered
+// with the kernel that reads it; the FFMA path takes them from the host.
+static int ddim_run(sdfb_ddpm* d, float* x_dev, const float* noise, int n, const std::vector<DdpmStep>& rows, int precision, cudaStream_t st,
+                    bool philox = false, unsigned long long seed = 0, unsigned int f0 = 0) {
+  const int steps = static_cast<int>(rows.size());
+  if (precision == SDFB_PREC_FP32) return sample_fp32(d, x_dev, noise, n, rows.data(), steps, st);
+  CU_TRY(cudaMemcpyAsync(d->call_rows_dev, rows.data(), rows.size() * sizeof(DdpmStep), cudaMemcpyHostToDevice, st));
+  return ddpm_tc(d, x_dev, noise, n, d->call_rows_dev, steps, nullptr, precision == SDFB_PREC_FP16, st, philox, seed, f0);
+}
+
+int sdfb_ddpm_sample_ddim(sdfb_ddpm* d, float* x_dev, const float* noise_dev, int n, int steps, float eta, int precision, void* stream) {
+  std::vector<DdpmStep> rows;
+  int rc = ddim_prepare(d, x_dev, n, steps, eta, 0, precision, rows);
+  if (rc) return rc;
+  if (eta > 0.f && !noise_dev) return fail(SDFB_E_INVALID, "noise stream required for eta > 0");
+  DeviceGuard g(d->device);
+  if (int prc = ddpm_pending_status(d)) return prc;
+  return ddim_run(d, x_dev, noise_dev, n, rows, precision, static_cast<cudaStream_t>(stream));
+}
+
+int sdfb_ddpm_sample_ddim_philox(sdfb_ddpm* d, float* x_dev, uint64_t seed, int64_t first_latent, int n, int steps, float eta, int gen_xT,
+                                 int precision, void* stream) {
+  std::vector<DdpmStep> rows;
+  int rc = ddim_prepare(d, x_dev, n, steps, eta, 0, precision, rows);
+  if (rc) return rc;
+  if (first_latent < 0 || first_latent + n > 0xFFFFFFFFll) return fail(SDFB_E_INVALID, "latent range outside [0, 2^32)");
+  const unsigned int f0 = static_cast<unsigned int>(first_latent);
+  DeviceGuard g(d->device);
+  if (int prc = ddpm_pending_status(d)) return prc;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // x_T = row t = 1000 of the stream whatever the step count: DDIM and the full DDPM chain start from the same x_T
+  if (gen_xT) CU_TRY(launch_philox_normal(seed, f0, n, kDdpmT, kDdpmT + 1, x_dev, st));
+  if (precision != SDFB_PREC_FP32) return ddim_run(d, x_dev, nullptr, n, rows, precision, st, true, seed, f0);
+  // fp32 path: materialise plane i = Philox row tau_i for the steps that draw noise, then run the FFMA sampler on it
+  const size_t cnt = static_cast<size_t>(n) * kDdpmLatent;
+  rc = ensure_stage(nullptr, nullptr, &d->nstage, &d->nstage_bytes, 0, static_cast<size_t>(steps) * cnt * sizeof(float));
+  if (rc) return rc;
+  float* nz = static_cast<float*>(d->nstage);
+  for (const DdpmStep& r : rows)
+    if (r.coef[5] != 0.f) CU_TRY(launch_philox_normal(seed, f0, n, r.t, r.t + 1, nz + static_cast<size_t>(r.plane) * cnt, st));
+  return ddim_run(d, x_dev, nz, n, rows, precision, st);
+}
+
+int sdfb_ddpm_invert_ddim(sdfb_ddpm* d, float* x_dev, int n, int steps, int precision, void* stream) {
+  std::vector<DdpmStep> rows;
+  int rc = ddim_prepare(d, x_dev, n, steps, 0.f, 1, precision, rows);
+  if (rc) return rc;
+  DeviceGuard g(d->device);
+  if (int prc = ddpm_pending_status(d)) return prc;
+  return ddim_run(d, x_dev, nullptr, n, rows, precision, static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

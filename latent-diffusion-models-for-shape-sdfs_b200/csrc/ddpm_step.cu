@@ -6,7 +6,9 @@
 //   per step t:  h0 = relu([x_hi | x_lo] [W0x | W0x]^T + tb0[t])      K = 512, time embedding folded
 //                h1..h3 = relu(h W^T + b)                             K = 1024
 //                eps = h3 W4^T + b4                                   fp32, never rounded
-//                x0 = clamp(sra x - srm1 eps, -1, 1);  x <- c1 x0 + c2 x + sigma noise[t]
+//                x0 = clamp(sra x - srm1 eps, -c, c);  x <- c1 x0 + c2 x [+ c3 eps] [+ sigma noise]
+//   with t, the noise plane and the coefficients read from the call's schedule table (DdpmStep, execution order):
+//   DDPM, DDIM sampling and DDIM inversion are different tables
 // 16-bit operands, fp32 accumulation in TMEM; the state x stays fp32 and enters layer 0 as an
 // exact two-way 16-bit split.
 //
@@ -21,7 +23,7 @@
 // only for the CTAs that share its 256 latents (one barrier counter per latent group: release-add
 // by the storing thread after its bulk stores completed, acquire spin in the producer); weights
 // do not depend on it and are prefetched across it.  The last layer's epilogue is the DDPM
-// update: x and noise[t] arrive as TMA boxes, x_new, x_hi and x_lo leave as TMA boxes.
+// update: x and the step's noise plane arrive as TMA boxes, x_new, x_hi and x_lo leave as TMA boxes.
 //
 //   warps 0-7  epilogue   (TMEM lane quadrant = warp & 3; the two warp sets split the columns)
 //   warp 8     producer   (TMA; completion counted on the LEADER's barrier)
@@ -463,9 +465,10 @@ ddpm_sample_kernel(const DdpmParams p, const __grid_constant__ CUtensorMap tm_ac
     const bool set_leader = (q == 0 && lane == 0);
     uint32_t acc_phase = 0, gt = 0, xn_phase = 0;
     for (int s = 0; s < p.steps; ++s) {
-      const int t = p.t_first - s;
-      const float4 cf = *reinterpret_cast<const float4*>(p.coef + t * 8);        // sra, srm1, c1, c2
-      const float sigma = p.coef[t * 8 + 4];
+      // this step's schedule row: the timestep here, the coefficients and the noise plane only in the last layer (kept out
+      // of the registers the hidden layers' epilogues need)
+      const DdpmStep* srow = p.sched + s;
+      const int t = srow->t;
       for (int l = 0; l < kLayers; ++l) {
         const Geo g = layer_geo(p, l);
         const float* bias = l == 0 ? p.tb0 + static_cast<long long>(t) * kDdpmHid
@@ -487,20 +490,26 @@ ddpm_sample_kernel(const DdpmParams p, const __grid_constant__ CUtensorMap tm_ac
           // waited for that before it got here).
           float* sb = sbias + (gt & 1u) * 256;
           if (static_cast<int>(threadIdx.x) < g.bn) sb[threadIdx.x] = bias[j * g.bn + threadIdx.x];
+          float4 cf = make_float4(0.f, 0.f, 0.f, 0.f), cg = cf;           // sra, srm1, c1, c2 | c3, sigma, clamp
+          if (l == 4) {
+            cf = reinterpret_cast<const float4*>(srow->coef)[0];
+            cg = reinterpret_cast<const float4*>(srow->coef)[1];
+          }
+          const float sigma = cg.y;
           named_bar_sync(1, kEpiThreads);
           if (l == 4 && threadIdx.x == 0 && !p.eps_mode) {
-            // x and noise[t] of this half tile: two 32-column fp32 boxes each
+            // x and this step's noise plane of this half tile: two 32-column fp32 boxes each
             const uint32_t xn = bars + 8 * kBarXn;
-            const bool nz_box = t > 0 && !p.philox;
+            const bool nz_box = sigma != 0.f && !p.philox;
             mbar_arrive_expect_tx(xn, (nz_box ? 4u : 2u) * kChunk);
             tma_load_2d(stg, &tm_x, j * 64, g_row, xn);
             tma_load_2d(stg + kChunk, &tm_x, j * 64 + 32, g_row, xn);
             if (nz_box) {
-              tma_load_3d(stg + 2 * kChunk, &tm_nz, j * 64, g_row, t, xn);
-              tma_load_3d(stg + 3 * kChunk, &tm_nz, j * 64 + 32, g_row, t, xn);
+              tma_load_3d(stg + 2 * kChunk, &tm_nz, j * 64, g_row, srow->plane, xn);
+              tma_load_3d(stg + 3 * kChunk, &tm_nz, j * 64 + 32, g_row, srow->plane, xn);
             }
           }
-          if (l == 4 && p.philox && !p.eps_mode && t > 0) {
+          if (l == 4 && p.philox && !p.eps_mode && sigma != 0.f) {
             // in-kernel noise: this thread's 32 normals -> its row of the noise box (the layout the TMA box would
             // have had), generated while the tensor core is still busy with this tile
             const uint32_t nrow_w = stg + (2 + set) * kChunk + row * 128u;
@@ -613,7 +622,7 @@ ddpm_sample_kernel(const DdpmParams p, const __grid_constant__ CUtensorMap tm_ac
             }
           } else {
             // last layer (64 features per tile; set s owns columns [32 s, 32 s + 32)):
-            // eps -> x0-clipped posterior-mean update, op for op as oracle/ddpm.py ddpm_step
+            // eps -> the schedule row's update, op for op as oracle/ddpm.py ddpm_step (DDPM rows) and tests/ddim_reference.py (DDIM rows)
             uint32_t v[32];
             tmem_ld32(tbase + set * 32, v);
             if (!p.eps_mode) {
@@ -636,7 +645,7 @@ ddpm_sample_kernel(const DdpmParams p, const __grid_constant__ CUtensorMap tm_ac
               for (int u = 0; u < 8; ++u) {
                 const uint32_t off = (static_cast<uint32_t>(u) ^ row7) << 4;
                 xq[u] = ld_shared_f4(xrow + off);
-                nq[u] = t > 0 ? ld_shared_f4(nrow + off) : make_float4(0.f, 0.f, 0.f, 0.f);
+                nq[u] = sigma != 0.f ? ld_shared_f4(nrow + off) : make_float4(0.f, 0.f, 0.f, 0.f);
               }
             }
             named_bar_sync(1, kEpiThreads);
@@ -658,9 +667,10 @@ ddpm_sample_kernel(const DdpmParams p, const __grid_constant__ CUtensorMap tm_ac
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
                   float x0 = __fsub_rn(__fmul_rn(cf.x, xs[e]), __fmul_rn(cf.y, ev[e]));
-                  x0 = fminf(fmaxf(x0, -1.f), 1.f);
+                  x0 = fminf(fmaxf(x0, -cg.z), cg.z);
                   r[e] = __fadd_rn(__fmul_rn(cf.z, x0), __fmul_rn(cf.w, xs[e]));
-                  if (t > 0) r[e] = __fadd_rn(r[e], __fmul_rn(sigma, ns[e]));
+                  if (cg.x != 0.f) r[e] = __fadd_rn(r[e], __fmul_rn(cg.x, ev[e]));
+                  if (sigma != 0.f) r[e] = __fadd_rn(r[e], __fmul_rn(sigma, ns[e]));
                 }
                 o = make_float4(r[0], r[1], r[2], r[3]);
                 split2<FP16>(r[0], r[1], hi[2 * (u & 1)], lo[2 * (u & 1)]);

@@ -363,16 +363,18 @@ __global__ void mask_pack_linear_kernel(const unsigned int* __restrict__ rowmask
 }
 
 // A7, op-for-op as the oracle evaluates it (separately rounded multiplies and adds).
+// The row format is DdpmStep::coef: sra, srm1, c1, c2, c3, sigma, clamp.
+struct UpdateCoef { float sra, srm1, c1, c2, c3, sigma, clamp; };
 __global__ void ddpm_update_kernel(float* __restrict__ x, const float* __restrict__ eps,
-                                   const float* __restrict__ noise, long long count, float sra,
-                                   float srm1, float c1, float c2, float sigma) {
+                                   const float* __restrict__ noise, long long count, const UpdateCoef c) {
   const long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
   if (i >= count) return;
-  const float xv = x[i];
-  float x0 = __fsub_rn(__fmul_rn(sra, xv), __fmul_rn(srm1, eps[i]));
-  x0 = fminf(fmaxf(x0, -1.f), 1.f);
-  float o = __fadd_rn(__fmul_rn(c1, x0), __fmul_rn(c2, xv));
-  if (noise) o = __fadd_rn(o, __fmul_rn(sigma, noise[i]));
+  const float xv = x[i], ev = eps[i];
+  float x0 = __fsub_rn(__fmul_rn(c.sra, xv), __fmul_rn(c.srm1, ev));
+  x0 = fminf(fmaxf(x0, -c.clamp), c.clamp);
+  float o = __fadd_rn(__fmul_rn(c.c1, x0), __fmul_rn(c.c2, xv));
+  if (c.c3 != 0.f) o = __fadd_rn(o, __fmul_rn(c.c3, ev));
+  if (c.sigma != 0.f) o = __fadd_rn(o, __fmul_rn(c.sigma, noise[i]));
   x[i] = o;
 }
 
@@ -500,12 +502,12 @@ cudaError_t launch_mask_from_bits(const unsigned int* bits, int nz, int ny, int 
   return e;
 }
 
-cudaError_t launch_ddpm_update(float* x, const float* eps, const float* noise, long long count,
-                               float sra, float srm1, float c1, float c2, float sigma,
+cudaError_t launch_ddpm_update(float* x, const float* eps, const float* noise, long long count, const float* coef,
                                cudaStream_t stream) {
   if (count <= 0) return cudaSuccess;
-  ddpm_update_kernel<<<blocks_for(count, 256), 256, 0, stream>>>(x, eps, noise, count, sra, srm1, c1, c2,
-                                                                sigma);
+  if (coef[5] != 0.f && noise == nullptr) return cudaErrorInvalidValue;
+  const UpdateCoef c{coef[0], coef[1], coef[2], coef[3], coef[4], coef[5], coef[6]};
+  ddpm_update_kernel<<<blocks_for(count, 256), 256, 0, stream>>>(x, eps, noise, count, c);
   return cudaGetLastError();
 }
 

@@ -131,15 +131,27 @@ constexpr int kDdpmMaxStages = 8;
 constexpr int kDdpmActCols = 512 + 1024 + 1024;
 constexpr int kDdpmOutTile = 64;          // output-layer tile width (fixed)
 
+// One row of a sampler schedule, in execution order.  The update of a step is
+//   x0 = clamp(sra x - srm1 eps, -clamp, clamp);  x <- c1 x0 + c2 x [+ c3 eps] [+ sigma noise]
+// (every product and sum rounded on its own; the c3 term only when c3 != 0, the noise term only when sigma != 0).
+// DDPM: c3 = 0, clamp = 1, noise plane = t.  DDIM sampling: plane = step index.  DDIM inversion: c3 != 0, sigma = 0,
+// clamp = +inf.
+struct DdpmStep {
+  float coef[8];           // sra, srm1, c1, c2, c3, sigma, clamp, 0   (the row format of sdfb_ddim_schedule)
+  int t;                   // timestep: the tb0 row and the Philox counter's step field
+  int plane;               // plane of the explicit noise stream
+  int pad[2];
+};
+static_assert(sizeof(DdpmStep) == 48, "DdpmStep is read as three 16-byte vectors");
+
 struct DdpmParams {
   const float* tb0;        // [1000][1024]: b0 + W0[:, 256:] temb(t)
   const float* bias;       // [3][1024] (layers 1-3) then [256] (layer 4)
-  const float* coef;       // [1000][8]: sra, srm1, c1, c2, sigma
+  const DdpmStep* sched;   // [steps]: the rows of this call, in execution order
   int eps_mode;            // 1: a single denoiser evaluation, eps_hat is stored through tm_x (no update)
   int n;
   int pair_m_tiles;        // ceil(n / 256)
-  int steps;               // steps to run: t = t_first, t_first - 1, ...
-  int t_first;
+  int steps;               // steps to run: sched[0], sched[1], ...
   int bn_h;                // output-tile width of the hidden layers (256, 128 or - small batches - 64)
   int nstages;
   int cluster8;            // 1: a cluster = the pair tiles of one latent group (one tile per pair and layer): the group barrier
@@ -163,7 +175,7 @@ struct DdpmMaps {
   alignas(64) unsigned char wh[128];    // weights, box 64 x bn_h / 2, no swizzle
   alignas(64) unsigned char wo[128];    // weights, box 64 x 32
   alignas(64) unsigned char x[128];     // fp32 state [n][256] (eps_mode: the eps output), box 32 x 128, SWIZZLE_128B
-  alignas(64) unsigned char nz[128];    // fp32 noise [steps][n][256], box 32 x 128 x 1, SWIZZLE_128B
+  alignas(64) unsigned char nz[128];    // fp32 noise [planes][n][256], box 32 x 128 x 1, SWIZZLE_128B
 };
 
 cudaError_t ddpm_step_init();
@@ -287,9 +299,8 @@ cudaError_t launch_sign_bits(const float* sdf, long long M, unsigned int* bits, 
 size_t mask_rows_words(int nz, int ny, int nx);
 cudaError_t launch_mask_from_bits(const unsigned int* bits, int nz, int ny, int nx, unsigned char* mask_u8,
                                   unsigned int* mask_bits, unsigned int* rowmask, cudaStream_t stream);
-// x <- c1*clamp(sra*x - srm1*eps, -1, 1) + c2*x + sigma*noise   (noise may be null)
-cudaError_t launch_ddpm_update(float* x, const float* eps, const float* noise, long long count,
-                               float sra, float srm1, float c1, float c2, float sigma,
+// the update of one DdpmStep row (coef = its first 8 floats): noise is used only when sigma != 0
+cudaError_t launch_ddpm_update(float* x, const float* eps, const float* noise, long long count, const float* coef,
                                cudaStream_t stream);
 
 // ---- marching cubes (marching.cu) --------------------------------------------

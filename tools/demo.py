@@ -2,7 +2,9 @@
 """End-to-end demo of the hot path on one GPU: sample latents with the fused DDPM kernel, decode one of them
 (or the synthetic default latent) on a res^3 grid, extract the zero level set and write it as a Wavefront OBJ.
 
-    python tools/demo.py [--res 128] [--out shape.obj] [--sampled] [--sparse] [--fit N]
+    python tools/demo.py [--res 128] [--out shape.obj] [--sampled [--ddim S]] [--sparse] [--fit N]
+
+--ddim S samples with S respaced DDIM steps (eta = 0) instead of the 1000-step DDPM chain.
 
 --fit N closes the loop: N SDF samples of the decoded shape are fitted by a FRESH latent (auto-decoder inference, one
 forward + backward launch of the fused kernel per Adam step) and the refitted shape is what gets meshed.
@@ -33,6 +35,7 @@ def main():
     ap.add_argument("--res", type=int, default=128)
     ap.add_argument("--out", default="shape.obj")
     ap.add_argument("--sampled", action="store_true", help="decode a latent drawn by the DDPM sampler instead of the synthetic one")
+    ap.add_argument("--ddim", type=int, default=0, metavar="S", help="with --sampled: S deterministic DDIM steps instead of 1000 DDPM steps")
     ap.add_argument("--sparse", action="store_true", help="sparse extraction (decode only near the surface)")
     ap.add_argument("--fit", type=int, default=0, metavar="N", help="refit the shape from N of its own SDF samples (tensor-pipe latent fitting)")
     ap.add_argument("--fit-steps", type=int, default=400)
@@ -42,8 +45,12 @@ def main():
     if args.sampled:
         ddpm = pkg.LatentDDPM(pkg.synthetic.ddpm_params(), precision="bf16")
         t0 = time.perf_counter()
-        z = ddpm.sample_latents(256, seed=1)[0]
-        print(f"sampled 256 latents in {ddpm.last_kernel_ms():.1f} ms (kernel), {1e3 * (time.perf_counter() - t0):.1f} ms (call)")
+        if args.ddim > 0:
+            z = ddpm.sample_latents_ddim(256, steps=args.ddim, eta=0.0, seed=1)[0]
+        else:
+            z = ddpm.sample_latents(256, seed=1)[0]
+        how = f"{args.ddim} DDIM steps" if args.ddim > 0 else "1000 DDPM steps"
+        print(f"sampled 256 latents ({how}) in {ddpm.last_kernel_ms():.1f} ms (kernel), {1e3 * (time.perf_counter() - t0):.1f} ms (call)")
     else:
         z = torch.from_numpy(pkg.synthetic.latent(0)).cuda()
     if args.fit > 0:
